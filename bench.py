@@ -25,6 +25,10 @@ SURVEY.md §8d) summed over the steps / time. Rank 0 prints ONE JSON line.
   sssp / other_configs   BASELINE configs 2-5 side runs (SSSP lines carry their own roofline block).
   --impl reference   times the reference's CPU implementation alone on the SAME graph and sources, one bfs_cpu per
                host thread (the only other place oracle/ is executed).
+  --dump-outputs DIR   after the timed steps, writes the depth array of the last timed BFS (what ess_bfs hands its
+               caller) to DIR/bfs_depth.npy, float64; above DUMP_SAMPLE vertices a fixed strided sample of positions,
+               listed in DIR/bfs_depth_index.npy. Graph and sources are seeded, so two builds run with the same
+               arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -67,7 +71,41 @@ def parse():
     ap.add_argument("--extras-budget-s", type=float, default=420.0,
                     help="side runs are skipped once the process has been running this long")
     ap.add_argument("--cpu-threads", type=int, default=0, help="reference arm: concurrent bfs_cpu runs (0 = auto)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the output of the last timed step as DIR/<name>.npy (see the module docstring)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_SAMPLE = 1 << 21  # entries kept per dumped output: 16 MiB of float64 values plus 16 MiB of positions
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each named tensor as out_dir/<name>.npy in float64 (exact for int32 depths and float32 distances). A
+    tensor longer than DUMP_SAMPLE keeps DUMP_SAMPLE positions at a fixed stride, the same for every run and every
+    install (graphgen permutes vertex ids, so a stride samples the graph evenly); the positions go to
+    out_dir/<name>_index.npy."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        n = t.numel()
+        if n > DUMP_SAMPLE:
+            idx = torch.arange(DUMP_SAMPLE, dtype=torch.int64) * (n // DUMP_SAMPLE)
+            vals = t[idx.to(t.device)]
+            np.save(os.path.join(out_dir, f"{name}_index.npy"), idx.numpy().astype(np.float64))
+        else:
+            vals = t
+        np.save(os.path.join(out_dir, f"{name}.npy"), vals.cpu().numpy().astype(np.float64))
+
+
+def check_sources(srcs, count):
+    """The timed loop runs one step per source: fewer sources than asked for would silently shorten it."""
+    if len(srcs) != count:
+        raise SystemExit(f"bench.py: the graph has only {len(srcs)} usable sources, {count} needed "
+                         f"(--steps + --warmup)")
 
 
 def peaks():
@@ -229,6 +267,7 @@ def run_reference(args, rank, world):
     dev = "cuda" if torch.cuda.is_available() else "cpu"
     csr = gg.rmat_csr(args.scale, args.edge_factor, device=dev)
     srcs = gg.pick_sources(csr, K + W)
+    check_sources(srcs, K + W)
     n, m = csr.n, csr.m
     off = csr.offsets.cpu().numpy()
     col = csr.indices.cpu().numpy()
@@ -263,6 +302,8 @@ def run_reference(args, rank, world):
         t0 = time.time()
         res = list(pool.map(work, srcs[W:]))
         wall = time.time() - t0
+    if args.dump_outputs:  # work() keeps no depth arrays (K of them would not fit at scale 26): rerun the last source
+        dump_outputs(args.dump_outputs, {"bfs_depth": torch.from_numpy(one(srcs[-1])[0])})
     edges = sum(r[0] for r in res)
     search_ms = sum(r[1] for r in res)
     val = edges / wall / 1e9
@@ -342,6 +383,7 @@ def run_single(args, rank, local_rank):
     stream.synchronize()
     n, m, offset_bits = csr.n, csr.m, graph.offset_bits
     srcs = gg.pick_sources(csr, K + W)
+    check_sources(srcs, K + W)
     timed = srcs[W:]
 
     def one_bfs(s, g=None):
@@ -377,6 +419,8 @@ def run_single(args, rank, local_rank):
     clocks = sampler.stop()
     launches = ctx.launches() - launches0
     value = edges / (ms * 1e-3) / 1e9
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"bfs_depth": depth})  # depth still holds the last timed source's BFS
 
     out = {
         "metric": "BFS GTEPS", "value": value, "unit": "GTEPS", "n_gpus": 1, "steps": K, "warmup": W,
@@ -650,13 +694,14 @@ def run_distributed(args, rank, world, local_rank):
         dist.all_reduce(t)
         return int(t.item())
 
-    def measure(scale, steps, warm, sssp_steps=0, check_single=False):
+    def measure(scale, steps, warm, sssp_steps=0, check_single=False, dump_dir=None):
         """One partitioned workload: timed BFS (and SSSP) steps + certificates. Returns a dict (same on every rank)."""
         runner = edist.build_partitioned(scale, args.edge_factor, rank, world, dev, stream,
                                          weights="hash" if sssp_steps else "none")
         stream.synchronize()
         with torch.cuda.stream(stream):
             srcs = runner.pick_sources(steps + warm)
+        check_sources(srcs, steps + warm)
         timed = srcs[warm:]
         work, viol = {}, 0
         with torch.cuda.stream(stream):
@@ -685,6 +730,13 @@ def run_distributed(args, rank, world, local_rank):
         torch.cuda.synchronize()
         dist.barrier()
         ms = all_max(e0.elapsed_time(e1))
+        if dump_dir:
+            with torch.cuda.stream(stream):
+                full = runner.gather_depth()  # collective: the last timed source's depths, all partitions
+            stream.synchronize()
+            if rank == 0:
+                dump_outputs(dump_dir, {"bfs_depth": full})
+            del full
         r = {"scale": scale, "n": runner.n_global, "m": runner.m_global, "offset_bits": runner.offset_bits,
              "steps": steps, "ms": ms, "edges": edges, "gteps": edges / (ms * 1e-3) / 1e9,
              "certificate_violations": viol, "launches": runner.backend.launches() - launches0,
@@ -771,7 +823,7 @@ def run_distributed(args, rank, world, local_rank):
         torch.cuda.empty_cache()
         return r
 
-    main = measure(args.scale, K, W, sssp_steps=2, check_single=True)
+    main = measure(args.scale, K, W, sssp_steps=2, check_single=True, dump_dir=args.dump_outputs)
     parity_ok = main["certificate_violations"] == 0 and main.get("equal_single_gpu_bfs", True) \
         and main.get("sssp", {}).get("certificate_violations", 0) == 0
     out = {

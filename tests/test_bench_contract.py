@@ -6,6 +6,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -30,6 +32,69 @@ def test_reference_arm_prints_one_contract_line():
     import bench
     assert d["config"] == bench.workload_config(12, 16, d["config"]["n"], d["config"]["m"], 2)
     assert d["scaling"] == "strong"
+
+
+def _bench_dump(tmp_path, run, *flags):
+    """Runs bench.py at scale 12 with --dump-outputs; returns (JSON line, dumped depth array, last timed source)."""
+    sys.path.insert(0, ROOT)
+    import numpy as np
+    from essentials_b200 import graphgen as gg
+    out_dir = str(tmp_path / f"dump{run}")
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--scale", "12", "--steps", "3", "--warmup",
+                          "1", "--dump-outputs", out_dir, *flags], capture_output=True, text=True, timeout=300, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-1500:]
+    assert sorted(os.listdir(out_dir)) == ["bfs_depth.npy"], "4096 vertices are below the sampling threshold"
+    depth = np.load(os.path.join(out_dir, "bfs_depth.npy"))
+    src = gg.pick_sources(gg.rmat_csr(12, 16), 4)[-1]
+    return json.loads(out.stdout.strip().splitlines()[-1]), depth, src
+
+
+def test_reference_arm_dumps_the_last_timed_bfs(tmp_path):
+    """--dump-outputs: the depths of the last timed source, float64, identical from run to run."""
+    import numpy as np
+    import oracle
+    from essentials_b200 import graphgen as gg
+    d, depth, src = _bench_dump(tmp_path, 0, "--impl", "reference")
+    assert d["steps"] == 3 and depth.dtype == np.float64
+    off, col, _ = gg.rmat_csr(12, 16).host()
+    assert np.array_equal(depth, oracle.bfs(off, col, src).astype(np.float64))
+    assert np.array_equal(_bench_dump(tmp_path, 1, "--impl", "reference")[1], depth)
+
+
+@pytest.mark.gpu
+def test_product_arm_dumps_the_last_timed_bfs(tmp_path):
+    import numpy as np
+    import oracle
+    from essentials_b200 import graphgen as gg
+    d, depth, src = _bench_dump(tmp_path, 0, "--no-extras", "--no-cpu", "--no-e2e")
+    assert d["steps"] == 3 and d["parity_ok"] is True
+    off, col, _ = gg.rmat_csr(12, 16).host()
+    assert np.array_equal(depth, oracle.bfs(off, col, src).astype(np.float64))
+
+
+def test_dump_of_a_long_output_is_a_fixed_sample(tmp_path):
+    """Above DUMP_SAMPLE entries (every scale-26 run): DUMP_SAMPLE values at fixed positions, listed beside them."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    n = bench.DUMP_SAMPLE * 3 + 5
+    depth = torch.randint(0, 2**31 - 1, (n,), dtype=torch.int32)
+    for run in (0, 1):
+        bench.dump_outputs(str(tmp_path / f"d{run}"), {"bfs_depth": depth})
+    vals, idx = (np.load(str(tmp_path / "d0" / f)) for f in ("bfs_depth.npy", "bfs_depth_index.npy"))
+    assert vals.dtype == idx.dtype == np.float64 and vals.size == idx.size == bench.DUMP_SAMPLE
+    assert vals.nbytes + idx.nbytes <= 64 * 2**20
+    assert np.all(np.diff(idx) > 0) and idx[0] >= 0 and idx[-1] < n
+    assert np.array_equal(vals, depth.numpy()[idx.astype(np.int64)].astype(np.float64))
+    for f in ("bfs_depth.npy", "bfs_depth_index.npy"):
+        assert np.array_equal(np.load(str(tmp_path / "d1" / f)), np.load(str(tmp_path / "d0" / f)))
+
+
+def test_steps_below_one_are_refused():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--scale", "10",
+                          "--steps", "0"], capture_output=True, text=True, timeout=300, cwd=ROOT)
+    assert out.returncode != 0 and not out.stdout.strip()
 
 
 def test_default_workload_is_the_north_star():
