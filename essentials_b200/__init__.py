@@ -34,6 +34,16 @@ class EssentialsError(RuntimeError):
     """Raised when a C-ABI call returns non-zero (mirrors gunrock::error::exception_t)."""
 
 
+class OutputOverflow(EssentialsError):
+    """An operator produced more elements than the caller's output buffer holds. `produced` is the full count,
+    `prefix` the `capacity` elements the buffer kept (which ones is unspecified, like the slot order), `calls` the
+    per-edge call counts of the run."""
+
+    def __init__(self, what: str, produced: int, capacity: int, prefix, calls):
+        super().__init__(f"{what}: produced {produced} elements, the output holds {capacity}")
+        self.produced, self.capacity, self.prefix, self.calls = produced, capacity, prefix, calls
+
+
 class RunInfo(Structure):
     _fields_ = [("enact_ms", c_float), ("iterations", c_int32), ("pull_steps", c_int32), ("push_steps", c_int32),
                 ("reserved", c_int64 * 8)]
@@ -376,36 +386,56 @@ def randoms(ctx: Context, n: int, begin: float, end: float, device="cuda"):
     return out
 
 
+def _frontier_edges(g: Graph, frontier, backward: bool) -> int:
+    """Σ out-degree (in-degree when `backward`) of the valid items of `frontier`: the most an advance can emit."""
+    import torch
+    view = g.csc if backward and g.csc is not None else g.csr
+    f = frontier.to(view.offsets.device, torch.int64)
+    f = f[f >= 0]
+    return int((view.offsets[f + 1] - view.offsets[f]).sum()) if f.numel() else 0
+
+
+def _probe_output(what: str, out, cap: int, produced: int, calls):
+    if produced > cap:
+        raise OutputOverflow(what, produced, cap, out[:cap], calls)
+    return out[:produced], calls
+
+
 def advance_probe(ctx: Context, g: Graph, frontier, lb: str = "merge_path", direction: str = "forward",
-                  modulus: int = 3, count_calls: bool = True):
+                  modulus: int = 3, count_calls: bool = True, capacity: int | None = None):
     """operators::advance::execute with the header's fixed test operator. Returns (kept neighbours, per-edge
-    call counts or None)."""
+    call counts or None).
+
+    `capacity` sizes the output buffer handed to the operator (default: the frontier's Σdeg + 1, which always fits).
+    A smaller buffer takes the operator's grow-and-relaunch path; if more neighbours are kept than it holds,
+    :class:`OutputOverflow` is raised with the produced count and the prefix that fits."""
     import torch
     _need_cuda(frontier)
     calls = torch.zeros(max(g.m, 1), dtype=torch.int32, device=frontier.device) if count_calls else None
     n_out = c_int64(0)
-    # first call sizes the output, second fills it — the probe operator is idempotent apart from `calls`
-    cap = int(g.m) + 1
-    out = torch.empty(cap, dtype=torch.int32, device=frontier.device)
+    cap = _frontier_edges(g, frontier, direction == "backward") + 1 if capacity is None else int(capacity)
+    out = torch.empty(max(cap, 1), dtype=torch.int32, device=frontier.device)
     _check(lib().ess_advance_probe(ctx.handle, g.handle, LOAD_BALANCE[lb], DIRECTION[direction], _p(frontier),
                                    int(frontier.numel()), _p(out), cap, byref(n_out), _p(calls), modulus),
            "ess_advance_probe")
-    return out[: n_out.value], calls
+    return _probe_output("ess_advance_probe", out, cap, n_out.value, calls)
 
 
-def advance_unique_probe(ctx: Context, g: Graph, frontier, lb: str = "merge_path", modulus: int = 3):
+def advance_unique_probe(ctx: Context, g: Graph, frontier, lb: str = "merge_path", modulus: int = 3,
+                         capacity: int | None = None):
     """operators::advance::execute_unique (fused advance + uniquify) with the fixed test operator, run twice on the
-    same bitmap. Returns (duplicate-free kept neighbours, per-edge call counts == 2 on every expanded edge)."""
+    same bitmap. Returns (duplicate-free kept neighbours, per-edge call counts == 2 on every expanded edge).
+    `capacity` as for :func:`advance_probe`; the operator's capacity guard still compares it with Σdeg."""
     import torch
     _need_cuda(frontier)
     calls = torch.zeros(max(g.m, 1), dtype=torch.int32, device=frontier.device)
     n_out = c_int64(0)
-    cap = int(g.m) + 1
-    out = torch.empty(cap, dtype=torch.int32, device=frontier.device)
+    cap = _frontier_edges(g, frontier, False) + 1 if capacity is None else int(capacity)
+    out = torch.empty(max(cap, 1), dtype=torch.int32, device=frontier.device)
     _check(lib().ess_advance_unique_probe(ctx.handle, g.handle, LOAD_BALANCE[lb], _p(frontier), int(frontier.numel()),
                                           _p(out), cap, byref(n_out), _p(calls), modulus),
            "ess_advance_unique_probe")
-    return out[: n_out.value], calls
+    return _probe_output("ess_advance_unique_probe", out, cap, n_out.value, calls)
 
 
 def filter_probe(ctx: Context, g: Graph, items, alg: str = "predicated", modulus: int = 3, in_place: bool = False):

@@ -618,6 +618,8 @@ static __global__ void __launch_bounds__(256)
     if (threadIdx.x < unsigned(world))
       s_dirty[threadIdx.x] = int(threadIdx.x) == rank ? 0u : reps.dirty[threadIdx.x][global_chunk];
     __syncthreads();
+    // float4 accesses: the replicas and dist_local are allocated by the dist handle itself (the peers' replicas
+    // through IPC), never by a caller, and row_begin and v0 are multiples of 1024 and 4
     const unsigned v0 = (c << 10) + threadIdx.x * 4;
     float4 best = *reinterpret_cast<const float4*>(replica_self + row_begin + v0);
     for (int p0 = 0; p0 < world; p0 += 8) {  // all fetches of a batch in flight before the first min

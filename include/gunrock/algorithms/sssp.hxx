@@ -247,12 +247,15 @@ __global__ void __launch_bounds__(256)
   __shared__ b200::counter_t sm[256 / 32 + 4];
   unsigned pending = 0, nearest = 0;
   const std::size_t per_cta = 256 * 4;
+  const bool vector_dist = (reinterpret_cast<std::uintptr_t>(dist) & 15u) == 0;
   for (std::size_t base = std::size_t(blockIdx.x) * per_cta; base < std::size_t(n);
        base += std::size_t(gridDim.x) * per_cta) {
     const std::size_t first = base + std::size_t(threadIdx.x) * 4;
     vertex_t ids[4];
     weight_t d[4], e[4];
-    if (first + 4 <= std::size_t(n) && sizeof(weight_t) == 4) {  // n-length arrays from cudaMalloc: 16-byte aligned
+    // `dist` is the caller's output array, possibly a tensor view at any 4-byte offset; `expanded` is run_delta's
+    // own n-length cudaMalloc'd array, 256-byte aligned
+    if (vector_dist && first + 4 <= std::size_t(n) && sizeof(weight_t) == 4) {
       const float4 a = *reinterpret_cast<const float4*>(dist + first);
       const float4 b = *reinterpret_cast<const float4*>(expanded + first);
       d[0] = a.x, d[1] = a.y, d[2] = a.z, d[3] = a.w;

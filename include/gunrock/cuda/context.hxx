@@ -65,7 +65,9 @@ struct scratch_t {
   unsigned long long* d = nullptr;  // device counters
   unsigned long long* h = nullptr;  // pinned host mirror
   memory::device_array_t<unsigned char> arena;
-  std::uint64_t max_degree_key = 0;  // cache: (offsets pointer ^ n) -> max degree
+  // cache: (graph build serial, offsets of the view) -> max degree of that view
+  std::uint64_t max_degree_graph = 0;
+  const void* max_degree_offsets = nullptr;
   long long max_degree_val = -1;
 
   scratch_t() = default;

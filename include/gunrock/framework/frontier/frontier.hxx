@@ -60,7 +60,7 @@ __global__ void __launch_bounds__(256) iota_kernel(type_t* out, std::size_t coun
   const std::size_t stride = std::size_t(gridDim.x) * blockDim.x;
   if constexpr (sizeof(type_t) == 4) {
     const std::size_t quads = count / 4;
-    int4* out4 = reinterpret_cast<int4*>(out);  // cudaMalloc'd base: 256-byte aligned
+    int4* out4 = reinterpret_cast<int4*>(out);  // only a frontier's own cudaMalloc'd base: 256-byte aligned
     for (std::size_t q = std::size_t(blockIdx.x) * blockDim.x + threadIdx.x; q < quads; q += stride) {
       int b = int(first) + int(q * 4);
       out4[q] = make_int4(b, b + 1, b + 2, b + 3);

@@ -46,18 +46,24 @@ using gcuda::scratch_t;
 using kernels::counter_t;
 using kernels::visit_t;
 
-/// Max degree of the adjacency, computed once per (context, offsets array) and cached.
+/// Max degree of one view of a graph, computed once per (context, graph build, view) and cached. The key is the
+/// graph's build serial, not the offsets address: a graph built over recycled memory (the torch caching allocator,
+/// the handle's device pool) must not inherit the max degree of the graph that lived there before, because a stale,
+/// too small value switches off the output-capacity guard of the thread- and block-mapped kernels. Serial 0 (a graph
+/// set() on the device) is never cached.
 template <typename vertex_t, typename edge_t>
-long long max_degree(gcuda::standard_context_t& ctx, const edge_t* offsets, vertex_t n) {
+long long max_degree(gcuda::standard_context_t& ctx, std::uint64_t graph_serial, const edge_t* offsets, vertex_t n) {
   auto& s = ctx.scratch();
-  const std::uint64_t key = std::uint64_t(reinterpret_cast<std::uintptr_t>(offsets)) ^ (std::uint64_t(n) << 1) ^ 1u;
-  if (s.max_degree_key == key && s.max_degree_val >= 0) return s.max_degree_val;
+  if (graph_serial != 0 && s.max_degree_graph == graph_serial && s.max_degree_offsets == offsets &&
+      s.max_degree_val >= 0)
+    return s.max_degree_val;
   auto stream = ctx.stream();
   cudaMemsetAsync(s.d + scratch_t::aux3, 0, sizeof(counter_t), stream);
   kernels::max_degree_kernel<<<gcuda::persistent_grid(ctx, (std::size_t(n) + 255) / 256, 8), 256, 0, stream>>>(
       offsets, n, s.d + scratch_t::aux3);
   s.fetch(stream);
-  s.max_degree_key = key;
+  s.max_degree_graph = graph_serial;
+  s.max_degree_offsets = offsets;
   s.max_degree_val = (long long)s.h[scratch_t::aux3];
   return s.max_degree_val;
 }
@@ -126,7 +132,7 @@ void expand(graph_t& G, operator_t op, frontier_t* input, frontier_t* output, wo
   long long maxdeg = 0;
   if constexpr (lb == load_balance_t::thread_mapped || lb == load_balance_t::block_mapped ||
                 lb == load_balance_t::merge_path || lb == load_balance_t::merge_path_v2)
-    maxdeg = max_degree(ctx, A.offsets, A.n);
+    maxdeg = max_degree(ctx, G.get_build_serial(), A.offsets, A.n);
   for (int attempt = 0; attempt < 3; ++attempt) {
     scratch.zero(stream);
     vertex_t* out = has_output ? output->data() : nullptr;
@@ -308,6 +314,10 @@ void expand(graph_t& G, operator_t op, frontier_t* input, frontier_t* output, wo
         grow_output(output, std::size_t(scratch.h[scratch_t::overflow]));
         continue;
       }
+      // every kernel drops stores past `capacity` but keeps counting: a count above it with no overflow flagged means
+      // the guard was skipped on a wrong max degree. The operator has run already, so a relaunch would call it twice
+      error::throw_if_exception(scratch.h[scratch_t::out_count] > capacity,
+                                "advance: output count exceeds the output capacity but no overflow was flagged");
       output->set_number_of_elements(std::size_t(scratch.h[scratch_t::out_count]));
     }
     return;

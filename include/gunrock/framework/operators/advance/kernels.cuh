@@ -421,6 +421,8 @@ __global__ void __launch_bounds__(cta_threads)
   __shared__ unsigned long long prefix[2];
   __shared__ int s_tile;
   const int n_tiles = int((input_size + per_tile - 1) / per_tile);
+  // the frontier may be a caller's buffer at any 4-byte offset (a tensor view): 128-bit loads need 16 bytes
+  const bool vector_input = (reinterpret_cast<std::uintptr_t>(input) & 15u) == 0;
   for (;;) {
     if (threadIdx.x == 0) s_tile = int(atomicAdd(counters + scratch_t::ticket, counter_t(1)));
     __syncthreads();
@@ -430,7 +432,7 @@ __global__ void __launch_bounds__(cta_threads)
     vertex_t v[prep_items];
     edge_t beg[prep_items], deg[prep_items];
     if constexpr (!graph_input) {
-      if (first + prep_items <= input_size && prep_items == 4 && sizeof(vertex_t) == 4) {
+      if (vector_input && first + prep_items <= input_size && prep_items == 4 && sizeof(vertex_t) == 4) {
         const int4 q = *reinterpret_cast<const int4*>(input + first);  // 128-bit frontier load
         v[0] = vertex_t(q.x), v[1] = vertex_t(q.y), v[2] = vertex_t(q.z), v[3] = vertex_t(q.w);
       } else {

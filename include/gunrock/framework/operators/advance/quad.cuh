@@ -56,7 +56,9 @@ inline int& advance_engine() {
 // 128-bit loads
 
 /// x[0..3] = p[e0..e0+3]; e0 is a multiple of 4 and p is 16-byte aligned. The last quad of an array whose length
-/// is not a multiple of 4 is read element-wise (no access past `count`).
+/// is not a multiple of 4 is read element-wise (no access past `count`). p is only ever a graph's column indices or
+/// values, and expand() takes the quad engine only after checking both on the host; graphs over arrays at another
+/// offset run the scalar kernels.
 template <typename T, typename index_t>
 __device__ __forceinline__ void load_quad(const T* __restrict__ p, index_t e0, index_t count, T (&x)[4]) {
   static_assert(sizeof(T) == 4, "quad loads move four 4-byte elements");
@@ -291,6 +293,8 @@ __global__ void __launch_bounds__(cta_threads)
   __shared__ unsigned long long prefix[2];
   __shared__ int s_tile;
   const int n_tiles = int((input_size + per_tile - 1) / per_tile);
+  // the frontier may be a caller's buffer at any 4-byte offset (a tensor view): 128-bit loads need 16 bytes
+  const bool vector_input = (reinterpret_cast<std::uintptr_t>(input) & 15u) == 0;
   for (;;) {
     if (threadIdx.x == 0) s_tile = int(atomicAdd(counters + scratch_t::ticket, counter_t(1)));
     __syncthreads();
@@ -300,7 +304,7 @@ __global__ void __launch_bounds__(cta_threads)
     vertex_t v[prep_items];
     edge_t beg[prep_items], end[prep_items];
     if constexpr (!graph_input) {
-      if (first + prep_items <= input_size && prep_items == 4 && sizeof(vertex_t) == 4) {
+      if (vector_input && first + prep_items <= input_size && prep_items == 4 && sizeof(vertex_t) == 4) {
         const int4 q = *reinterpret_cast<const int4*>(input + first);  // 128-bit frontier load
         v[0] = vertex_t(q.x), v[1] = vertex_t(q.y), v[2] = vertex_t(q.z), v[3] = vertex_t(q.w);
       } else {
@@ -824,7 +828,7 @@ __global__ void __launch_bounds__(cta_threads, 4)
         if (k < cur.n_quads) {
           have |= 1u << q;
           if (4 * k + 4 <= cur.covered) {
-            const int4 x = *reinterpret_cast<const int4*>(&s_col[stage][4 * k]);
+            const int4 x = *reinterpret_cast<const int4*>(&s_col[stage][4 * k]);  // shared-memory stage, 16-B aligned
             c[0] = vertex_t(x.x), c[1] = vertex_t(x.y), c[2] = vertex_t(x.z), c[3] = vertex_t(x.w);
           } else {
             load_quad(A.indices, e0[q], A.m, c);  // ragged last quad of the array

@@ -37,10 +37,17 @@ constexpr int cta_threads = 256;
 constexpr int items = 4;
 constexpr int per_tile = cta_threads * items;
 
+/// 16-byte alignment of a 128-bit access. Filter inputs and outputs are caller buffers, which may be tensor views
+/// at any element offset.
+template <typename type_t>
+__device__ __forceinline__ bool vector_aligned(const type_t* p) {
+  return (reinterpret_cast<std::uintptr_t>(p) & 15u) == 0;
+}
+
 template <typename type_t>
 __device__ __forceinline__ void load_items(const type_t* __restrict__ in, std::size_t first, std::size_t count,
                                            type_t (&v)[items]) {
-  if (sizeof(type_t) == 4 && first + items <= count) {
+  if (sizeof(type_t) == 4 && first + items <= count && vector_aligned(in)) {
     const int4 q = *reinterpret_cast<const int4*>(in + first);
     v[0] = type_t(q.x), v[1] = type_t(q.y), v[2] = type_t(q.z), v[3] = type_t(q.w);
   } else {
@@ -168,7 +175,7 @@ __global__ void __launch_bounds__(cta_threads)
 #pragma unroll
     for (int k = 0; k < items; ++k)
       if (gunrock::util::limits::is_valid(v[k]) && !op(v[k])) v[k] = gunrock::numeric_limits<type_t>::invalid();
-    if (sizeof(type_t) == 4 && first + items <= count) {
+    if (sizeof(type_t) == 4 && first + items <= count && vector_aligned(out)) {
       *reinterpret_cast<int4*>(out + first) = make_int4(int(v[0]), int(v[1]), int(v[2]), int(v[3]));
     } else {
 #pragma unroll

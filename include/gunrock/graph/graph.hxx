@@ -16,6 +16,7 @@
  */
 #pragma once
 
+#include <atomic>
 #include <cstdint>
 #include <tuple>
 #include <type_traits>
@@ -62,6 +63,12 @@ struct empty_csc_t {};
 struct empty_coo_t {};
 
 namespace detail {
+/// Process-wide counter behind graph_t::get_build_serial(); never returns 0.
+inline std::uint64_t next_build_serial() {
+  static std::atomic<std::uint64_t> serial{0};
+  return serial.fetch_add(1, std::memory_order_relaxed) + 1;
+}
+
 /// Largest row r with offsets[r] <= e, skipping empty rows: the row that owns edge e.
 template <typename vertex_t, typename edge_t>
 __host__ __device__ __forceinline__ vertex_t owner_of_edge(const edge_t* offsets, vertex_t rows, edge_t e) {
@@ -372,7 +379,15 @@ class graph_t : public graph_view_t... {
   template <class input_view_t = default_view_t, typename... args_t>
   __host__ __device__ void set(vertex_t const& n, edge_t const& m, args_t... args) {
     input_view_t::set(n, m, args...);
+#ifndef __CUDA_ARCH__
+    build_serial = detail::next_build_serial();
+#endif
   }
+
+  /// Identity of the arrays this graph was last set() over, unique within the process (0: set on the device, or
+  /// never). Copies of a graph share it. Host caches of per-graph facts key on it rather than on array addresses,
+  /// which allocators hand out again once a graph's arrays are freed.
+  std::uint64_t get_build_serial() const { return build_serial; }
 
   template <typename input_view_t = default_view_t>
   __host__ __device__ __forceinline__ edge_t get_number_of_neighbors(vertex_t const& v) const {
@@ -405,6 +420,7 @@ class graph_t : public graph_view_t... {
 
  private:
   graph_properties_t properties;
+  std::uint64_t build_serial = 0;
 };
 
 /// Raw adjacency triple handed to the advance kernels (offsets, indices, values) for one view.
