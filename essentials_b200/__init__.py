@@ -76,6 +76,8 @@ _SIGNATURES = {
                                        c_void_p]),
     "ess_transpose_csr": (c_int, [c_int64, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "ess_bfs": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_int, c_int, c_float, c_float, POINTER(RunInfo)]),
+    "ess_bfs_tree": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_int, c_int, c_float, c_float,
+                             POINTER(RunInfo)]),
     "ess_sssp": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_int, POINTER(RunInfo)]),
     "ess_sssp_near_far": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_float, POINTER(RunInfo)]),
     "ess_sssp_delta": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_float, POINTER(RunInfo)]),
@@ -293,6 +295,34 @@ def bfs(ctx: Context, g: Graph, source: int, lb: str = "block_mapped", direction
     _check(lib().ess_bfs(ctx.handle, g.handle, int(source), _p(depth), LOAD_BALANCE[lb], DIRECTION[direction],
                          alpha, beta, byref(info)), "ess_bfs")
     return depth, info.as_dict()
+
+
+def _label_buffer(t, g: Graph, what: str):
+    import torch
+    if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.int32 and t.is_contiguous()
+            and t.numel() >= g.n and t.device == g.device):
+        raise EssentialsError(f"{what} must be a contiguous int32 CUDA tensor of at least {g.n} elements on {g.device}")
+    return t
+
+
+def bfs_tree(ctx: Context, g: Graph, source: int, lb: str = "block_mapped", direction: str = "forward", out=None,
+             pred_out=None, alpha: float = 0.0, beta: float = 0.0):
+    """gunrock::bfs::run_tree: :func:`bfs` plus the BFS tree. Returns (depth[int32], pred[int32], info).
+
+    `depth` and `info` are what :func:`bfs` returns. pred[source] == source; pred[v] == -1 exactly where v is unreached
+    (depth INT32_MAX); every other pred[v] is an in-neighbour u of v (an edge u -> v) with depth[u] == depth[v] - 1.
+    Which valid parent is chosen is not deterministic. `out` and `pred_out`, when given, must be contiguous int32 CUDA
+    tensors of at least g.n elements on the graph's device, and must not overlap."""
+    import torch
+    depth = _out(g.n, torch.int32, g) if out is None else _label_buffer(out, g, "out")
+    pred = _out(g.n, torch.int32, g) if pred_out is None else _label_buffer(pred_out, g, "pred_out")
+    span = 4 * g.n
+    if depth.data_ptr() < pred.data_ptr() + span and pred.data_ptr() < depth.data_ptr() + span:
+        raise EssentialsError("bfs_tree: pred_out must not overlap out")
+    info = RunInfo()
+    _check(lib().ess_bfs_tree(ctx.handle, g.handle, int(source), _p(depth), _p(pred), LOAD_BALANCE[lb],
+                              DIRECTION[direction], alpha, beta, byref(info)), "ess_bfs_tree")
+    return depth, pred, info.as_dict()
 
 
 def sssp(ctx: Context, g: Graph, source: int, lb: str = "block_mapped", out=None):

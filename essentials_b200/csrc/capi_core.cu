@@ -49,7 +49,7 @@ int& host_chunk_edges() {
 extern "C" {
 
 const char* ess_last_error(void) { return ess::last_error().c_str(); }
-int ess_version(void) { return 100; }
+int ess_version(void) { return 101; }
 
 int ess_context_create(int device, void* stream, int own_stream, ess_context_t* out) {
   ESS_TRY

@@ -120,6 +120,16 @@ ESS_API int ess_transpose_csr(int64_t n, int64_t m, int offset_bits, const void*
 ESS_API int ess_bfs(ess_context_t ctx, ess_graph_t g, int32_t source, int32_t* d_depth, int lb, int direction,
             float alpha, float beta, ess_run_info* info);
 
+/* gunrock::bfs::run_tree: ess_bfs plus the BFS tree. d_depth, the arguments and info are exactly as for ess_bfs.
+ * d_pred: n x int32, 4-byte aligned, required, must not alias d_depth. On return:
+ *   d_pred[source] == source;
+ *   d_pred[v] == -1 if and only if d_depth[v] == INT32_MAX (v unreached);
+ *   otherwise 0 <= d_pred[v] < n, the CSR holds an edge d_pred[v] -> v, and d_depth[d_pred[v]] == d_depth[v] - 1.
+ * Which of several valid parents is chosen depends on scheduling and is not deterministic. Every entry is written, so
+ * what d_pred held before the call does not matter. */
+ESS_API int ess_bfs_tree(ess_context_t ctx, ess_graph_t g, int32_t source, int32_t* d_depth, int32_t* d_pred, int lb,
+                         int direction, float alpha, float beta, ess_run_info* info);
+
 /* gunrock::sssp::run — include/gunrock/algorithms/sssp.hxx:155-185. d_dist: n x float, FLT_MAX = unreachable. */
 ESS_API int ess_sssp(ess_context_t ctx, ess_graph_t g, int32_t source, float* d_dist, int lb, ess_run_info* info);
 

@@ -9,6 +9,8 @@
  *   bfs::run(G, src, dist, pred)                                   == reference behaviour (block_mapped push)
  *   bfs::run<load_balance_t::merge_path, advance_direction_t::optimized>(...)  = push/pull switching
  * Depths are an order-independent fixed point, so every variant returns the same array.
+ * run_tree() takes the same arguments and also writes the BFS tree into `predecessors` (DESIGN.md §3.5); run() never
+ * touches that array, so callers that size it arbitrarily (the reference's drivers pass a 1-element vector) stay safe.
  * With a partitioned context (gcuda::partition_t, one process per GPU) the same loop body runs on the owned rows and
  * operators::exchange::execute routes each level's discoveries to their owners: `distances` is then a full-length
  * array whose owned slice is the result.
@@ -29,12 +31,15 @@ struct param_t {
 template <typename vertex_t>
 struct result_t {
   vertex_t* distances;
-  vertex_t* predecessors;  ///< accepted for signature parity; not produced (the reference leaves it a todo)
+  vertex_t* predecessors;  ///< written by run_tree() only; run() accepts it for signature parity and leaves it alone
   result_t(vertex_t* _distances, vertex_t* _predecessors) : distances(_distances), predecessors(_predecessors) {}
 };
 
-template <typename graph_t, typename param_type, typename result_type>
+/// `tree`: also record each reached vertex's parent in result.predecessors (run_tree). The depth-only problem and its
+/// enactor instantiate exactly the operators they always had.
+template <typename graph_t, typename param_type, typename result_type, bool tree = false>
 struct problem_t : gunrock::problem_t<graph_t> {
+  static constexpr bool record_tree = tree;
   param_type param;
   result_type result;
   using vertex_t = typename graph_t::vertex_type;
@@ -60,6 +65,26 @@ struct problem_t : gunrock::problem_t<graph_t> {
     cudaMemsetAsync(settled.data(), 0, settled.size() * sizeof(unsigned), ctx->stream());
     b200::set_one(*ctx, settled.data() + (std::size_t(param.single_source) >> 5),
                   1u << (unsigned(param.single_source) & 31u));
+    if constexpr (tree) {  // -1 = unreached; the source is its own parent
+      b200::fill(*ctx, result.predecessors, n, vertex_t(-1));
+      b200::set_one(*ctx, result.predecessors + param.single_source, param.single_source);
+    }
+  }
+};
+
+/// A BFS operator that also records the parent: it returns true for exactly one call per vertex (push: the caller whose
+/// atomic::min lowered the depth from INT_MAX; bottom-up and claim-first top-down: the thread that owns the vertex), so
+/// that call stores `source` as the vertex's parent with a plain store and no other call touches it.
+template <typename op_t, typename vertex_t>
+struct record_parent_t {
+  op_t op;
+  vertex_t* predecessors;
+  template <typename edge_t, typename weight_t>
+  __host__ __device__ __forceinline__ bool operator()(vertex_t const& source, vertex_t const& neighbor,
+                                                      edge_t const& edge, weight_t const& weight) const {
+    if (!op(source, neighbor, edge, weight)) return false;
+    predecessors[neighbor] = source;
+    return true;
   }
 };
 
@@ -90,6 +115,13 @@ struct enactor_t : gunrock::enactor_t<problem_t> {
     auto P = this->get_problem();
     auto G = P->get_graph();
     auto distances = P->result.distances;
+    // the depth-only problem gets its operators back unchanged
+    auto with_parent = [P](auto op) {
+      if constexpr (problem_t::record_tree)
+        return record_parent_t<decltype(op), vertex_t>{op, P->result.predecessors};
+      else
+        return op;
+    };
     const vertex_t next_depth = vertex_t(this->iteration + 1);
 
     unsigned* settled = P->settled.data();
@@ -117,9 +149,10 @@ struct enactor_t : gunrock::enactor_t<problem_t> {
         distances[neighbor] = next_depth;
         return true;
       };
-      operators::advance::execute<lb, direction>(G, E, operators::advance::directional(search, adopt), context);
+      operators::advance::execute<lb, direction>(
+          G, E, operators::advance::directional(with_parent(search), with_parent(adopt)), context);
     } else {
-      operators::advance::execute<lb, direction>(G, E, search, context);
+      operators::advance::execute<lb, direction>(G, E, with_parent(search), context);
     }
     if (context.partition && context.partition->world > 1) {
       // 1-D partitioned run: discovered vertices go to their owners, who keep min(depth) and de-duplicate
@@ -130,18 +163,15 @@ struct enactor_t : gunrock::enactor_t<problem_t> {
   }
 };
 
-template <operators::load_balance_t lb = operators::load_balance_t::block_mapped,
-          operators::advance_direction_t direction = operators::advance_direction_t::forward, typename graph_t>
+namespace detail {
+template <bool tree, operators::load_balance_t lb, operators::advance_direction_t direction, typename graph_t>
 float run(graph_t& G, typename graph_t::vertex_type& single_source, typename graph_t::vertex_type* distances,
-          typename graph_t::vertex_type* predecessors,
-          std::shared_ptr<gcuda::multi_context_t> context =
-              std::shared_ptr<gcuda::multi_context_t>(new gcuda::multi_context_t(0)),
-          enactor_properties_t properties = enactor_properties_t(), int* pull_steps = nullptr, int* iterations = nullptr,
-          long long* work_stats = nullptr) {
+          typename graph_t::vertex_type* predecessors, std::shared_ptr<gcuda::multi_context_t> context,
+          enactor_properties_t properties, int* pull_steps, int* iterations, long long* work_stats) {
   using vertex_t = typename graph_t::vertex_type;
   using param_type = param_t<vertex_t>;
   using result_type = result_t<vertex_t>;
-  using problem_type = problem_t<graph_t, param_type, result_type>;
+  using problem_type = problem_t<graph_t, param_type, result_type, tree>;
   using enactor_type = enactor_t<problem_type, lb, direction>;
 
   param_type param(single_source);
@@ -163,6 +193,43 @@ float run(graph_t& G, typename graph_t::vertex_type& single_source, typename gra
     work_stats[6] = enactor.direction.push_vertices_found;  // [6] vertices claimed top-down
   }
   return ms;
+}
+}  // namespace detail
+
+/// Depths only: `predecessors` is accepted for signature parity with the reference and never read or written.
+template <operators::load_balance_t lb = operators::load_balance_t::block_mapped,
+          operators::advance_direction_t direction = operators::advance_direction_t::forward, typename graph_t>
+float run(graph_t& G, typename graph_t::vertex_type& single_source, typename graph_t::vertex_type* distances,
+          typename graph_t::vertex_type* predecessors,
+          std::shared_ptr<gcuda::multi_context_t> context =
+              std::shared_ptr<gcuda::multi_context_t>(new gcuda::multi_context_t(0)),
+          enactor_properties_t properties = enactor_properties_t(), int* pull_steps = nullptr, int* iterations = nullptr,
+          long long* work_stats = nullptr) {
+  return detail::run<false, lb, direction>(G, single_source, distances, predecessors, context, properties, pull_steps,
+                                           iterations, work_stats);
+}
+
+/**
+ * @brief run() plus the BFS tree. `distances` are the same as run()'s; `predecessors` (n entries, required, not
+ * aliasing `distances`) receives predecessors[source] = source, -1 for every unreached vertex, and for every other
+ * reached v an in-neighbour u (an edge u -> v of the CSR) with distances[u] == distances[v] - 1. Which of several such
+ * parents is chosen depends on scheduling. Every entry is written, whatever the array held before. Not available on a
+ * partitioned context: the exchange carries (vertex, depth) records only, so the parent would be lost at the owner.
+ */
+template <operators::load_balance_t lb = operators::load_balance_t::block_mapped,
+          operators::advance_direction_t direction = operators::advance_direction_t::forward, typename graph_t>
+float run_tree(graph_t& G, typename graph_t::vertex_type& single_source, typename graph_t::vertex_type* distances,
+               typename graph_t::vertex_type* predecessors,
+               std::shared_ptr<gcuda::multi_context_t> context =
+                   std::shared_ptr<gcuda::multi_context_t>(new gcuda::multi_context_t(0)),
+               enactor_properties_t properties = enactor_properties_t(), int* pull_steps = nullptr,
+               int* iterations = nullptr, long long* work_stats = nullptr) {
+  error::throw_if_exception(predecessors == nullptr, "bfs::run_tree: predecessors is required");
+  error::throw_if_exception(predecessors == distances, "bfs::run_tree: predecessors must not alias distances");
+  error::throw_if_exception(context->partition && context->partition->world > 1,
+                            "bfs::run_tree: the BFS tree is not available on a partitioned context");
+  return detail::run<true, lb, direction>(G, single_source, distances, predecessors, context, properties, pull_steps,
+                                          iterations, work_stats);
 }
 
 }  // namespace bfs
