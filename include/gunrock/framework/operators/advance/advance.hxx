@@ -82,16 +82,224 @@ void grow_output(frontier_t* output, std::size_t needed) {
   if (output->get_capacity() < needed) output->reserve(needed);
 }
 
-/**
- * @brief Push-direction expansion with one of the balancers. `visited` non-null selects the
- * test-and-set policy (direction-optimised callers); null keeps reference semantics.
- * `input_size_on_device`/`next_edges` are used by the optimised path only.
- */
 struct no_epilogue_t {
   template <typename... args_t>
   void operator()(args_t&&...) const {}
 };
 
+/// Calls f(std::true_type{}) or f(std::false_type{}), so that a runtime flag picks a kernel's template flag in
+/// one launch expression.
+template <typename F>
+void with_bool(bool b, F&& f) {
+  if (b)
+    f(std::true_type{});
+  else
+    f(std::false_type{});
+}
+
+/**
+ * @brief The push kernels of one expansion attempt, one launcher per balancer. Each launcher chooses once between
+ * the quad engine (quad.cuh) and the scalar kernels, and brackets its launches for the profiler.
+ */
+template <bool graph_input, bool has_output, visit_t policy, typename vertex_t, typename edge_t, typename weight_t,
+          typename operator_t>
+struct push_launch_t {
+  /// 128-bit column / weight loads need 4-byte elements (and 16-byte aligned arrays, checked at run time)
+  static constexpr bool quad_types = sizeof(vertex_t) == 4 && sizeof(weight_t) == 4;
+
+  gcuda::standard_context_t& ctx;
+  graph::adjacency_t<vertex_t, edge_t, weight_t> A;
+  operator_t& op;
+  const vertex_t* in;
+  std::size_t nf;
+  vertex_t* out;
+  counter_t* C;
+  counter_t capacity;
+  unsigned* visited;
+  bool quad;  // the quad engine runs (never true without quad_types)
+  long long maxdeg;
+
+  gcuda::profiler_t& prof() { return ctx.profiler(); }
+  gcuda::stream_t stream() { return ctx.stream(); }
+  std::size_t item_ctas() const { return (nf + kernels::cta_threads - 1) / kernels::cta_threads; }
+
+  /// Calls f(std::bool_constant<quad>{}); the quad kernels are only instantiated for quad_types.
+  template <typename F>
+  void with_engine(F&& f) {
+    if constexpr (quad_types) {
+      if (quad) return f(std::true_type{});
+    }
+    f(std::false_type{});
+  }
+
+  /// Σdeg of the frontier, needed by the thread- and block-mapped kernels' capacity guard when every item at the
+  /// max degree might not fit the output. Returns whether the guard is on.
+  bool degree_sum_for_guard() {
+    const bool guard = has_output && (long double)(nf) * (long double)(maxdeg) > (long double)(capacity);
+    if (guard) {
+      prof().begin(gcuda::profiler_t::work_prepare, stream());
+      kernels::degree_sum_kernel<graph_input><<<gcuda::persistent_grid(ctx, item_ctas(), 8), 256, 0, stream()>>>(
+          A.offsets, in, nf, C);
+      prof().end(stream());
+    }
+    return guard;
+  }
+
+  /// The hubs deferred to `big_list` (block_mapped, bucketing), expanded grid-wide. The guard of these kernels
+  /// reads Σdeg, which is 0 = "fits" when it was not computed.
+  template <bool quad_engine>
+  void hubs(vertex_t* big_list) {
+    if constexpr (quad_engine) {  // column indices staged through shared memory by the TMA unit
+      auto kernel = kernels::big_list_bulk_kernel<has_output, policy, vertex_t, edge_t, weight_t, operator_t>;
+      kernel<<<gcuda::full_grid(ctx, kernel), 256, 0, stream()>>>(A, op, big_list, C + scratch_t::big_count, out, C,
+                                                                  capacity, visited);
+    } else {
+      kernels::big_list_kernel<has_output, policy>
+          <<<gcuda::persistent_grid(ctx, ~std::size_t(0), 6), 256, 0, stream()>>>(
+              A, op, big_list, C + scratch_t::big_count, out, C, capacity, visited);
+    }
+  }
+
+  void thread_mapped() {
+    const bool guard = degree_sum_for_guard();
+    prof().begin(gcuda::profiler_t::push_expand, stream());
+    with_bool(guard, [&](auto g) {
+      kernels::thread_mapped_kernel<graph_input, has_output, decltype(g)::value, policy>
+          <<<gcuda::persistent_grid(ctx, item_ctas(), 8), 256, 0, stream()>>>(A, op, in, nf, nullptr, out, C, capacity,
+                                                                              visited);
+    });
+    prof().end(stream());
+  }
+
+  void block_mapped() {
+    const bool guard = degree_sum_for_guard();
+    prof().begin(gcuda::profiler_t::push_expand, stream());
+    vertex_t* big_list = nullptr;
+    if (maxdeg >= kernels::big_degree) {
+      // a frontier may repeat a hub (SSSP), so the only safe bound on deferred items is nf
+      big_list = reinterpret_cast<vertex_t*>(ctx.scratch().temp(nf * sizeof(vertex_t)));
+    }
+    with_engine([&](auto q) {
+      with_bool(guard, [&](auto g) {
+        constexpr bool guarded = decltype(g)::value;
+        if constexpr (decltype(q)::value) {
+          auto kernel = kernels::block_mapped_quad_kernel<graph_input, has_output, guarded, policy, vertex_t, edge_t,
+                                                          weight_t, operator_t>;
+          kernel<<<gcuda::full_grid(ctx, kernel, item_ctas()), 256, 0, stream()>>>(A, op, in, nf, out, C, capacity,
+                                                                                   visited, big_list);
+        } else {
+          kernels::block_mapped_kernel<graph_input, has_output, guarded, policy>
+              <<<gcuda::persistent_grid(ctx, item_ctas(), 6), 256, 0, stream()>>>(A, op, in, nf, out, C, capacity,
+                                                                                  visited, big_list);
+        }
+      });
+      if (big_list) {
+        hubs<decltype(q)::value>(big_list);
+        prof().launches_total += 1;
+      }
+    });
+    prof().end(stream());
+  }
+
+  template <typename work_tiles_t>
+  void merge_path(work_tiles_t& segments) {
+    // CTAs the single-launch kernels can use on a tiny level
+    const long double bound = (long double)nf * (long double)maxdeg / kernels::tile_edges + 1;
+    const std::size_t tiles = bound > 1e9L ? std::size_t(1000000000) : std::size_t(bound);
+    with_engine([&](auto q) {
+      constexpr bool quad_engine = decltype(q)::value;
+      if (nf <= std::size_t(quad_engine ? kernels::small_items : kernels::tile_edges)) {
+        // tiny level: one launch, table built per CTA
+        prof().begin(gcuda::profiler_t::push_expand, stream());
+        if constexpr (quad_engine) {
+          auto kernel = kernels::merge_path_small_quad_kernel<graph_input, has_output, policy, vertex_t, edge_t,
+                                                              weight_t, operator_t>;
+          kernel<<<gcuda::full_grid(ctx, kernel, (tiles + 1) / 2), 256, 0, stream()>>>(A, op, in, int(nf), out, C,
+                                                                                       capacity, visited);
+        } else {
+          kernels::merge_path_small_kernel<graph_input, has_output, policy>
+              <<<gcuda::persistent_grid(ctx, tiles, 6), 256, 0, stream()>>>(A, op, in, int(nf), out, C, capacity,
+                                                                            visited);
+        }
+        prof().end(stream());
+        return;
+      }
+      if (segments.size() < nf + 1) segments.resize(nf + 1);
+      const std::size_t prep_tiles = (nf + kernels::cta_threads * kernels::prep_items - 1) /
+                                     (kernels::cta_threads * kernels::prep_items);
+      gcuda::arena_layout_t layout;
+      const std::size_t at_src = layout.add((nf + 1) * sizeof(vertex_t));
+      const std::size_t at_beg = layout.add((nf + 1) * sizeof(edge_t));
+      const std::size_t at_end = layout.add((nf + 1) * sizeof(edge_t));
+      const std::size_t at_state = layout.add(2 * prep_tiles * sizeof(b200::tile_word_t));
+      unsigned char* base = ctx.scratch().temp(layout.bytes);
+      auto* work_src = reinterpret_cast<vertex_t*>(base + at_src);
+      auto* work_beg = reinterpret_cast<edge_t*>(base + at_beg);
+      auto* work_end = reinterpret_cast<edge_t*>(base + at_end);
+      auto* state = reinterpret_cast<b200::tile_word_t*>(base + at_state);
+      edge_t* work_seg = raw_of(segments.data());
+      const unsigned prep_grid = gcuda::persistent_grid(ctx, prep_tiles, 6);
+      prof().begin(gcuda::profiler_t::work_prepare, stream());
+      cudaMemsetAsync(state, 0, 2 * prep_tiles * sizeof(b200::tile_word_t), stream());
+      if constexpr (quad_engine)
+        kernels::prepare_quads_kernel<graph_input><<<prep_grid, 256, 0, stream()>>>(
+            A.offsets, in, nf, work_src, work_beg, work_end, work_seg, state, state + prep_tiles, C);
+      else
+        kernels::prepare_work_kernel<graph_input><<<prep_grid, 256, 0, stream()>>>(
+            A.offsets, in, nf, work_src, work_beg, work_seg, state, state + prep_tiles, C);
+      prof().end(stream());
+      prof().begin(gcuda::profiler_t::push_expand, stream());
+      if constexpr (quad_engine) {
+        auto kernel = kernels::merge_path_quad_kernel<has_output, policy, vertex_t, edge_t, weight_t, operator_t>;
+        kernel<<<gcuda::full_grid(ctx, kernel), 256, 0, stream()>>>(A, op, work_src, work_beg, work_end, work_seg, out,
+                                                                    C, capacity, visited);
+      } else {
+        kernels::merge_path_kernel<has_output, policy>
+            <<<gcuda::persistent_grid(ctx, ~std::size_t(0), 6), 256, 0, stream()>>>(A, op, work_src, work_beg,
+                                                                                    work_seg, out, C, capacity, visited);
+      }
+      prof().end(stream());
+    });
+  }
+
+  void bucketing() {
+    gcuda::arena_layout_t layout;
+    const std::size_t at_small = layout.add(nf * sizeof(vertex_t));
+    const std::size_t at_warp = layout.add(nf * sizeof(vertex_t));
+    const std::size_t at_big = layout.add(nf * sizeof(vertex_t));
+    unsigned char* base = ctx.scratch().temp(layout.bytes);
+    auto* small_list = reinterpret_cast<vertex_t*>(base + at_small);
+    auto* warp_list = reinterpret_cast<vertex_t*>(base + at_warp);
+    auto* big_list = reinterpret_cast<vertex_t*>(base + at_big);
+    prof().begin(gcuda::profiler_t::work_prepare, stream());
+    kernels::bin_by_degree_kernel<graph_input><<<gcuda::persistent_grid(ctx, item_ctas(), 8), 256, 0, stream()>>>(
+        A.offsets, in, nf, small_list, warp_list, big_list, C);
+    prof().end(stream());
+    prof().begin(gcuda::profiler_t::push_expand, stream());
+    kernels::thread_mapped_kernel<false, has_output, true, policy>
+        <<<gcuda::persistent_grid(ctx, item_ctas(), 8), 256, 0, stream()>>>(A, op, small_list, 0, C + scratch_t::aux0,
+                                                                            out, C, capacity, visited);
+    with_engine([&](auto q) {
+      if constexpr (decltype(q)::value) {
+        auto kernel = kernels::warp_mapped_quad_kernel<has_output, policy, vertex_t, edge_t, weight_t, operator_t>;
+        kernel<<<gcuda::full_grid(ctx, kernel, (nf + 7) / 8), 256, 0, stream()>>>(A, op, warp_list, C + scratch_t::aux1,
+                                                                                  out, C, capacity, visited);
+      } else {
+        kernels::warp_mapped_kernel<has_output, policy>
+            <<<gcuda::persistent_grid(ctx, (nf + 7) / 8, 8), 256, 0, stream()>>>(A, op, warp_list, C + scratch_t::aux1,
+                                                                                out, C, capacity, visited);
+      }
+      hubs<decltype(q)::value>(big_list);
+    });
+    prof().end(stream(), 3);
+  }
+};
+
+/**
+ * @brief Push-direction expansion with one of the balancers. `visited` non-null selects the
+ * test-and-set policy (direction-optimised callers); null keeps reference semantics.
+ * `epilogue(counters, output)` enqueues extra kernels that consume the device-side output count before the one sync.
+ */
 template <load_balance_t lb, bool use_csc, advance_io_type_t input_type, advance_io_type_t output_type, visit_t policy,
           typename graph_t, typename operator_t, typename frontier_t, typename work_tiles_t,
           typename epilogue_t = no_epilogue_t>
@@ -99,12 +307,14 @@ void expand(graph_t& G, operator_t op, frontier_t* input, frontier_t* output, wo
             gcuda::standard_context_t& ctx, unsigned* visited, epilogue_t epilogue = epilogue_t()) {
   using vertex_t = typename graph_t::vertex_type;
   using edge_t = typename graph_t::edge_type;
+  using weight_t = typename graph_t::weight_type;
   constexpr bool graph_input = input_type == advance_io_type_t::graph;
   constexpr bool has_output = output_type != advance_io_type_t::none;
   static_assert(input_type == advance_io_type_t::graph || input_type == advance_io_type_t::vertices,
                 "advance input must be `graph` or `vertices`");
   static_assert(output_type == advance_io_type_t::none || output_type == advance_io_type_t::vertices,
                 "advance output must be `vertices` or `none`");
+  using launch_t = push_launch_t<graph_input, has_output, policy, vertex_t, edge_t, weight_t, operator_t>;
 
   const auto A = graph::adjacency_of<use_csc>(G);
   const std::size_t nf = graph_input ? std::size_t(A.n) : input->get_number_of_elements();
@@ -113,17 +323,8 @@ void expand(graph_t& G, operator_t op, frontier_t* input, frontier_t* output, wo
     return;
   }
   auto& scratch = ctx.scratch();
-  auto& prof = ctx.profiler();
-  using gcuda::profiler_t;
   auto stream = ctx.stream();
-  const vertex_t* in = graph_input ? nullptr : input->data();
-  const std::size_t prep_tiles = (nf + kernels::cta_threads * kernels::prep_items - 1) /
-                                 (kernels::cta_threads * kernels::prep_items);
-  const std::size_t item_ctas = (nf + kernels::cta_threads - 1) / kernels::cta_threads;
-  // quad engine (quad.cuh): 128-bit column / weight loads need 4-byte elements and 16-byte aligned arrays
-  using weight_t = typename graph_t::weight_type;
-  constexpr bool quad_types = sizeof(vertex_t) == 4 && sizeof(weight_t) == 4;
-  const bool quad = quad_types && kernels::advance_engine() != 0 &&
+  const bool quad = launch_t::quad_types && kernels::advance_engine() != 0 &&
                     (reinterpret_cast<std::uintptr_t>(A.indices) & 15u) == 0 &&
                     (reinterpret_cast<std::uintptr_t>(A.values) & 15u) == 0;
 
@@ -133,175 +334,27 @@ void expand(graph_t& G, operator_t op, frontier_t* input, frontier_t* output, wo
   if constexpr (lb == load_balance_t::thread_mapped || lb == load_balance_t::block_mapped ||
                 lb == load_balance_t::merge_path || lb == load_balance_t::merge_path_v2)
     maxdeg = max_degree(ctx, G.get_build_serial(), A.offsets, A.n);
+  // merge_path over `input = graph` (PageRank push, SpMV): the frontier is every vertex in id order, so the
+  // scan + compaction pass of merge-path (16-24 bytes written and re-read per vertex) buys nothing over
+  // block-mapped tiles of 256 consecutive rows with dynamic tickets and hub deferral; same operator calls
+  constexpr bool as_block_mapped =
+      lb == load_balance_t::block_mapped ||
+      ((lb == load_balance_t::merge_path || lb == load_balance_t::merge_path_v2) && graph_input && launch_t::quad_types);
   for (int attempt = 0; attempt < 3; ++attempt) {
     scratch.zero(stream);
-    vertex_t* out = has_output ? output->data() : nullptr;
-    const counter_t capacity = has_output ? counter_t(output->get_capacity()) : counter_t(0);
-    counter_t* C = scratch.d;
-
-    // merge_path over `input = graph` (PageRank push, SpMV): the frontier is every vertex in id order, so the
-    // scan + compaction pass of merge-path (16-24 bytes written and re-read per vertex) buys nothing over
-    // block-mapped tiles of 256 consecutive rows with dynamic tickets and hub deferral; same operator calls
-    constexpr bool as_block_mapped =
-        lb == load_balance_t::block_mapped ||
-        ((lb == load_balance_t::merge_path || lb == load_balance_t::merge_path_v2) && graph_input && quad_types);
-    if constexpr (lb == load_balance_t::thread_mapped || as_block_mapped) {
-      const bool guard = has_output && (long double)(nf) * (long double)(maxdeg) > (long double)(capacity);
-      if (guard) {
-        prof.begin(profiler_t::work_prepare, stream);
-        kernels::degree_sum_kernel<graph_input><<<gcuda::persistent_grid(ctx, item_ctas, 8), 256, 0, stream>>>(
-            A.offsets, in, nf, C);
-        prof.end(stream);
-      }
-      prof.begin(profiler_t::push_expand, stream);
-      if constexpr (lb == load_balance_t::thread_mapped) {
-        const unsigned grid = gcuda::persistent_grid(ctx, item_ctas, 8);
-        if (guard)
-          kernels::thread_mapped_kernel<graph_input, has_output, true, policy>
-              <<<grid, 256, 0, stream>>>(A, op, in, nf, nullptr, out, C, capacity, visited);
-        else
-          kernels::thread_mapped_kernel<graph_input, has_output, false, policy>
-              <<<grid, 256, 0, stream>>>(A, op, in, nf, nullptr, out, C, capacity, visited);
-      } else {
-        vertex_t* big_list = nullptr;
-        if (maxdeg >= kernels::big_degree) {
-          // a frontier may repeat a hub (SSSP), so the only safe bound on deferred items is nf
-          big_list = reinterpret_cast<vertex_t*>(scratch.temp(nf * sizeof(vertex_t)));
-        }
-        if constexpr (quad_types) {
-          if (quad) {
-            if (guard) {
-              auto kernel = kernels::block_mapped_quad_kernel<graph_input, has_output, true, policy, vertex_t, edge_t,
-                                                              weight_t, operator_t>;
-              kernel<<<gcuda::full_grid(ctx, kernel, item_ctas), 256, 0, stream>>>(A, op, in, nf, out, C, capacity,
-                                                                                   visited, big_list);
-            } else {
-              auto kernel = kernels::block_mapped_quad_kernel<graph_input, has_output, false, policy, vertex_t, edge_t,
-                                                              weight_t, operator_t>;
-              kernel<<<gcuda::full_grid(ctx, kernel, item_ctas), 256, 0, stream>>>(A, op, in, nf, out, C, capacity,
-                                                                                   visited, big_list);
-            }
-            if (big_list) {  // hubs: column indices staged through shared memory by the TMA unit
-              auto kernel = kernels::big_list_bulk_kernel<has_output, policy, vertex_t, edge_t, weight_t, operator_t>;
-              kernel<<<gcuda::full_grid(ctx, kernel), 256, 0, stream>>>(A, op, big_list, C + scratch_t::big_count, out,
-                                                                        C, capacity, visited);
-              prof.launches_total += 1;
-            }
-          }
-        }
-        if (!quad) {
-          const unsigned grid = gcuda::persistent_grid(ctx, item_ctas, 6);
-          if (guard)
-            kernels::block_mapped_kernel<graph_input, has_output, true, policy>
-                <<<grid, 256, 0, stream>>>(A, op, in, nf, out, C, capacity, visited, big_list);
-          else
-            kernels::block_mapped_kernel<graph_input, has_output, false, policy>
-                <<<grid, 256, 0, stream>>>(A, op, in, nf, out, C, capacity, visited, big_list);
-          if (big_list) {
-            // (the hub kernel's capacity guard reads Σdeg, which is 0 = "fits" when it was not needed)
-            kernels::big_list_kernel<has_output, policy>
-                <<<gcuda::persistent_grid(ctx, ~std::size_t(0), 6), 256, 0, stream>>>(
-                    A, op, big_list, C + scratch_t::big_count, out, C, capacity, visited);
-            prof.launches_total += 1;
-          }
-        }
-      }
-      prof.end(stream);
-    } else if constexpr (lb == load_balance_t::merge_path || lb == load_balance_t::merge_path_v2) {
-      const std::size_t small_limit = quad ? std::size_t(kernels::small_items) : std::size_t(kernels::tile_edges);
-      if (nf <= small_limit) {  // tiny level: one launch, table built per CTA
-        long double bound = (long double)nf * (long double)maxdeg / kernels::tile_edges + 1;
-        const std::size_t tiles = bound > 1e9L ? std::size_t(1000000000) : std::size_t(bound);
-        prof.begin(profiler_t::push_expand, stream);
-        if constexpr (quad_types) {
-          if (quad) {
-            auto kernel = kernels::merge_path_small_quad_kernel<graph_input, has_output, policy, vertex_t, edge_t,
-                                                                weight_t, operator_t>;
-            kernel<<<gcuda::full_grid(ctx, kernel, (tiles + 1) / 2), 256, 0, stream>>>(A, op, in, int(nf), out, C,
-                                                                                       capacity, visited);
-          }
-        }
-        if (!quad)
-          kernels::merge_path_small_kernel<graph_input, has_output, policy>
-              <<<gcuda::persistent_grid(ctx, tiles, 6), 256, 0, stream>>>(A, op, in, int(nf), out, C, capacity,
-                                                                          visited);
-        prof.end(stream);
-      } else {
-        if (segments.size() < nf + 1) segments.resize(nf + 1);
-        gcuda::arena_layout_t layout;
-        const std::size_t at_src = layout.add((nf + 1) * sizeof(vertex_t));
-        const std::size_t at_beg = layout.add((nf + 1) * sizeof(edge_t));
-        const std::size_t at_end = layout.add((nf + 1) * sizeof(edge_t));
-        const std::size_t at_state = layout.add(2 * prep_tiles * sizeof(b200::tile_word_t));
-        unsigned char* base = scratch.temp(layout.bytes);
-        auto* work_src = reinterpret_cast<vertex_t*>(base + at_src);
-        auto* work_beg = reinterpret_cast<edge_t*>(base + at_beg);
-        auto* work_end = reinterpret_cast<edge_t*>(base + at_end);
-        auto* state = reinterpret_cast<b200::tile_word_t*>(base + at_state);
-        edge_t* work_seg = raw_of(segments.data());
-        prof.begin(profiler_t::work_prepare, stream);
-        cudaMemsetAsync(state, 0, 2 * prep_tiles * sizeof(b200::tile_word_t), stream);
-        if (quad)
-          kernels::prepare_quads_kernel<graph_input><<<gcuda::persistent_grid(ctx, prep_tiles, 6), 256, 0, stream>>>(
-              A.offsets, in, nf, work_src, work_beg, work_end, work_seg, state, state + prep_tiles, C);
-        else
-          kernels::prepare_work_kernel<graph_input><<<gcuda::persistent_grid(ctx, prep_tiles, 6), 256, 0, stream>>>(
-              A.offsets, in, nf, work_src, work_beg, work_seg, state, state + prep_tiles, C);
-        prof.end(stream);
-        prof.begin(profiler_t::push_expand, stream);
-        if constexpr (quad_types) {
-          if (quad) {
-            auto kernel = kernels::merge_path_quad_kernel<has_output, policy, vertex_t, edge_t, weight_t, operator_t>;
-            kernel<<<gcuda::full_grid(ctx, kernel), 256, 0, stream>>>(A, op, work_src, work_beg, work_end, work_seg,
-                                                                      out, C, capacity, visited);
-          }
-        }
-        if (!quad)
-          kernels::merge_path_kernel<has_output, policy>
-              <<<gcuda::persistent_grid(ctx, ~std::size_t(0), 6), 256, 0, stream>>>(A, op, work_src, work_beg, work_seg,
-                                                                                    out, C, capacity, visited);
-        prof.end(stream);
-      }
-    } else if constexpr (lb == load_balance_t::bucketing) {
-      gcuda::arena_layout_t layout;
-      const std::size_t at_small = layout.add(nf * sizeof(vertex_t));
-      const std::size_t at_warp = layout.add(nf * sizeof(vertex_t));
-      const std::size_t at_big = layout.add(nf * sizeof(vertex_t));
-      unsigned char* base = scratch.temp(layout.bytes);
-      auto* small_list = reinterpret_cast<vertex_t*>(base + at_small);
-      auto* warp_list = reinterpret_cast<vertex_t*>(base + at_warp);
-      auto* big_list = reinterpret_cast<vertex_t*>(base + at_big);
-      prof.begin(profiler_t::work_prepare, stream);
-      kernels::bin_by_degree_kernel<graph_input><<<gcuda::persistent_grid(ctx, item_ctas, 8), 256, 0, stream>>>(
-          A.offsets, in, nf, small_list, warp_list, big_list, C);
-      prof.end(stream);
-      prof.begin(profiler_t::push_expand, stream);
-      kernels::thread_mapped_kernel<false, has_output, true, policy>
-          <<<gcuda::persistent_grid(ctx, item_ctas, 8), 256, 0, stream>>>(A, op, small_list, 0, C + scratch_t::aux0, out,
-                                                                        C, capacity, visited);
-      if constexpr (quad_types) {
-        if (quad) {
-          auto warp_kernel = kernels::warp_mapped_quad_kernel<has_output, policy, vertex_t, edge_t, weight_t, operator_t>;
-          warp_kernel<<<gcuda::full_grid(ctx, warp_kernel, (nf + 7) / 8), 256, 0, stream>>>(
-              A, op, warp_list, C + scratch_t::aux1, out, C, capacity, visited);
-          auto hub_kernel = kernels::big_list_bulk_kernel<has_output, policy, vertex_t, edge_t, weight_t, operator_t>;
-          hub_kernel<<<gcuda::full_grid(ctx, hub_kernel), 256, 0, stream>>>(A, op, big_list, C + scratch_t::big_count,
-                                                                            out, C, capacity, visited);
-        }
-      }
-      if (!quad) {
-        kernels::warp_mapped_kernel<has_output, policy>
-            <<<gcuda::persistent_grid(ctx, (nf + 7) / 8, 8), 256, 0, stream>>>(A, op, warp_list, C + scratch_t::aux1, out,
-                                                                              C, capacity, visited);
-        kernels::big_list_kernel<has_output, policy>
-            <<<gcuda::persistent_grid(ctx, ~std::size_t(0), 6), 256, 0, stream>>>(
-                A, op, big_list, C + scratch_t::big_count, out, C, capacity, visited);
-      }
-      prof.end(stream, 3);
-    } else {
+    launch_t launch{ctx, A, op, graph_input ? nullptr : input->data(), nf, has_output ? output->data() : nullptr,
+                    scratch.d, has_output ? counter_t(output->get_capacity()) : counter_t(0), visited, quad, maxdeg};
+    if constexpr (lb == load_balance_t::thread_mapped)
+      launch.thread_mapped();
+    else if constexpr (as_block_mapped)
+      launch.block_mapped();
+    else if constexpr (lb == load_balance_t::merge_path || lb == load_balance_t::merge_path_v2)
+      launch.merge_path(segments);
+    else if constexpr (lb == load_balance_t::bucketing)
+      launch.bucketing();
+    else
       error::throw_if_exception(cudaErrorUnknown, "Advance type not supported.");
-    }
-    epilogue(C, out);  // extra kernels that consume the device-side output count before the one sync
+    epilogue(launch.C, launch.out);
     error::check_last("advance launch");
     if constexpr (!has_output)
       if (scratch.async_when_no_output) {  // nothing to report; the next zero() must really clear the counters
@@ -316,7 +369,7 @@ void expand(graph_t& G, operator_t op, frontier_t* input, frontier_t* output, wo
       }
       // every kernel drops stores past `capacity` but keeps counting: a count above it with no overflow flagged means
       // the guard was skipped on a wrong max degree. The operator has run already, so a relaunch would call it twice
-      error::throw_if_exception(scratch.h[scratch_t::out_count] > capacity,
+      error::throw_if_exception(scratch.h[scratch_t::out_count] > launch.capacity,
                                 "advance: output count exceeds the output capacity but no overflow was flagged");
       output->set_number_of_elements(std::size_t(scratch.h[scratch_t::out_count]));
     }
@@ -445,7 +498,8 @@ void optimized(graph_t& G, enactor_type* E, operator_t op, gcuda::standard_conte
     grow_output(output, std::size_t(n));
     // Σdeg of the new frontier (Beamer's m_f): one parallel pass over the output list, enqueued behind the
     // expansion kernels and in front of the level's single host round trip (it reads the list length from the
-    // device counter the expansion just produced).
+    // device counter the expansion just produced). It is not summed inside the expansion kernels: that put two
+    // dependent row-bound loads at the end of every discovery's probe -> test-and-set -> operator chain.
     const auto* degree_offsets = out_adj.offsets;
     auto degree_sum = [&](counter_t* C, vertex_t* out) {
       kernels::mark_frontier_kernel<<<gcuda::persistent_grid(ctx, ~std::size_t(0), 4), 256, 0, stream>>>(

@@ -8,9 +8,11 @@
  * (advance/block_mapped.hxx:38-147,155-205; advance/helpers.hxx:39-146; advance/thread_mapped.hxx:32-96;
  * advance/merge_path.hxx:35-114 = mgpu::transform_lbs).
  *
- * Here every balancer funnels into the same two device routines:
- *   - visit_edge():   load neighbour (read-only path), optional visited-bitmap pre-check (1 bit/vertex, L2
- *                     resident), call the user operator exactly once with lvalues, optional test-and-set.
+ * Every balancer of both engines (these scalar kernels and the quad engine of quad.cuh) applies the same
+ * visited-bitmap policy (1 bit/vertex, L2 resident), defined below: is_visited / drop_visited probe it,
+ * admit() claims a neighbour the operator kept, claim_first() claims a batch before the operator runs.
+ * The scalar kernels expand edges through two device routines:
+ *   - visit_edge():   probe, call the user operator exactly once with lvalues, admit.
  *   - expand_tile():  a CTA walks a tile of edges described by shared-memory (source, first edge, offset)
  *                     triples; ITEMS independent column loads per thread are issued before any operator
  *                     runs; survivors are compacted with ONE global atomic per CTA round (warp shuffle
@@ -55,41 +57,73 @@ constexpr int warp_degree = 32;                       // bucketing: lists at lea
 /// only by the first edge that sets its bit in the (per-call, initially clear) bitmap.
 enum class visit_t { none, test_and_set, unique_output };
 
-/// Σdeg of the vertices a test_and_set advance claims (Beamer's m_f of the next frontier) used to be accumulated
-/// inside the expansion kernels: two dependent random row-bound loads at the END of every discovery's chain
-/// (probe -> test-and-set -> operator), which ncu showed as the long-scoreboard tail of the heavy top-down level.
-/// It is now a separate, fully parallel pass over the output list (mark_frontier_kernel, enqueued by
-/// detail::optimized before the level's one host round trip).
-constexpr bool count_fresh_edges_in_kernel = false;
+// ------------------------------------------------------------------------------------------------
+// The visited-bitmap policy, shared by the scalar and quad engines.
 
-/// `fresh_edges` (test_and_set only) accumulates the out-degree of every vertex this thread adds to the
-/// visited set: Σdeg of the next frontier is Beamer's m_f, needed by the push/pull switch.
+__device__ __forceinline__ bool is_visited(unsigned* __restrict__ visited, unsigned v) {
+  return (visited[v >> 5] >> (v & 31u)) & 1u;
+}
+
+/// Sets v's bit; true iff this call set it.
+__device__ __forceinline__ bool test_and_set(unsigned* __restrict__ visited, unsigned v) {
+  const unsigned bit = 1u << (v & 31u);
+  return !(atomicOr(&visited[v >> 5], bit) & bit);
+}
+
+/// Clears the live bits of the items whose neighbour is already visited. All probes are issued before any is
+/// tested, so their round trips overlap.
+template <int N, typename vertex_t>
+__device__ __forceinline__ unsigned drop_visited(const vertex_t (&nbr)[N], unsigned live,
+                                                 unsigned* __restrict__ visited) {
+  unsigned word[N];
+#pragma unroll
+  for (int i = 0; i < N; ++i)
+    if (live & (1u << i)) word[i] = visited[unsigned(nbr[i]) >> 5];
+#pragma unroll
+  for (int i = 0; i < N; ++i)
+    if ((live & (1u << i)) && ((word[i] >> (unsigned(nbr[i]) & 31u)) & 1u)) live &= ~(1u << i);
+  return live;
+}
+
+/// After the operator: whether a neighbour it kept (`keep`) goes to the output. test_and_set admits the edge that
+/// claims the neighbour's bit; unique_output likewise, behind a plain read that keeps repeats off the atomic units.
+template <visit_t policy>
+__device__ __forceinline__ bool admit(unsigned* __restrict__ visited, unsigned neighbor, bool keep) {
+  if constexpr (policy == visit_t::test_and_set) {
+    if (keep) keep = test_and_set(visited, neighbor);
+  }
+  if constexpr (policy == visit_t::unique_output) {
+    if (keep) keep = !is_visited(visited, neighbor) && test_and_set(visited, neighbor);
+  }
+  return keep;
+}
+
+/// Claim-first test_and_set of a thread's N edges, for operators with an owner-exclusive (pull) form: probe all,
+/// then test-and-set the unvisited, so the dependent memory round trips of the discoveries overlap instead of
+/// running one after the other (ncu showed the heavy top-down levels long-scoreboard bound at 19 % issue
+/// utilisation with the per-edge chain, profiles/r01c_merge_path_heavy_push.txt). Returns the items whose
+/// neighbour this thread claimed; the caller runs the pull form of the operator on exactly those.
+template <int N, typename vertex_t>
+__device__ __forceinline__ unsigned claim_first(const vertex_t (&nbr)[N], unsigned live,
+                                                unsigned* __restrict__ visited) {
+  live = drop_visited(nbr, live, visited);
+  unsigned claimed = 0;
+#pragma unroll
+  for (int i = 0; i < N; ++i)
+    if ((live & (1u << i)) && test_and_set(visited, unsigned(nbr[i]))) claimed |= 1u << i;
+  return claimed;
+}
+
 template <visit_t policy, typename vertex_t, typename edge_t, typename weight_t, typename operator_t>
 __device__ __forceinline__ bool visit_edge(const graph::adjacency_t<vertex_t, edge_t, weight_t>& A,
                                            operator_t& op, vertex_t source, edge_t edge, vertex_t neighbor,
-                                           unsigned* __restrict__ visited, counter_t& fresh_edges) {
+                                           unsigned* __restrict__ visited) {
   if constexpr (policy == visit_t::test_and_set) {
-    if ((visited[unsigned(neighbor) >> 5] >> (unsigned(neighbor) & 31u)) & 1u) return false;
+    if (is_visited(visited, unsigned(neighbor))) return false;
   }
   weight_t weight = A.values ? __ldg(A.values + edge) : weight_t(1);
   source += A.source_offset;  // 1-D partition: operators see global vertex ids
-  bool keep = op(source, neighbor, edge, weight);
-  if constexpr (policy == visit_t::test_and_set) {
-    if (keep) {
-      const unsigned bit = 1u << (unsigned(neighbor) & 31u);
-      keep = !(atomicOr(&visited[unsigned(neighbor) >> 5], bit) & bit);
-      if constexpr (count_fresh_edges_in_kernel)
-        if (keep) fresh_edges += counter_t(A.offsets[neighbor + 1] - A.offsets[neighbor]);
-    }
-  }
-  if constexpr (policy == visit_t::unique_output) {
-    if (keep) {
-      const unsigned bit = 1u << (unsigned(neighbor) & 31u);
-      unsigned* word = &visited[unsigned(neighbor) >> 5];
-      keep = !(*word & bit) && !(atomicOr(word, bit) & bit);  // the plain read keeps repeats off the atomic units
-    }
-  }
-  return keep;
+  return admit<policy>(visited, unsigned(neighbor), op(source, neighbor, edge, weight));
 }
 
 /// unique_output epilogue: clears the bitmap words of the emitted vertices (only emitted vertices ever set a bit,
@@ -101,16 +135,6 @@ __global__ void __launch_bounds__(256)
        i += std::size_t(gridDim.x) * blockDim.x) {
     const vertex_t v = output[i];
     if (util::limits::is_valid(v)) seen[unsigned(v) >> 5] = 0u;
-  }
-}
-
-/// End-of-kernel flush of a thread's fresh_edges into counters[aux2] (one atomic per warp).
-template <visit_t policy>
-__device__ __forceinline__ void flush_fresh_edges(counter_t fresh_edges, counter_t* counters) {
-  if constexpr (policy == visit_t::test_and_set && count_fresh_edges_in_kernel) {
-    __syncwarp();
-    fresh_edges = b200::warp_sum(fresh_edges);
-    if (b200::lane_id() == 0 && fresh_edges) atomicAdd(counters + scratch_t::aux2, fresh_edges);
   }
 }
 
@@ -135,8 +159,7 @@ template <bool has_output, visit_t policy, typename vertex_t, typename edge_t, t
 __device__ __forceinline__ void expand_tile(const graph::adjacency_t<vertex_t, edge_t, weight_t>& A, operator_t& op,
                                             tile_smem_t<vertex_t, edge_t>& sm, int n_seg, edge_t n_edges,
                                             vertex_t* __restrict__ output, counter_t* counters, counter_t capacity,
-                                            unsigned* __restrict__ visited, counter_t& fresh_edges,
-                                            edge_t edge_base = 0) {
+                                            unsigned* __restrict__ visited, edge_t edge_base = 0) {
   // edge_base: when the segment table covers more than this tile (small-frontier kernel), tile edge r is
   // edge (edge_base + r) of the table.
   for (edge_t round = 0; round < n_edges; round += tile_edges) {
@@ -160,44 +183,18 @@ __device__ __forceinline__ void expand_tile(const graph::adjacency_t<vertex_t, e
       if (live & (1u << i)) nbr[i] = __ldg(A.indices + eid[i]);
     unsigned keep = 0;
     if constexpr (policy == visit_t::test_and_set && has_pull_operator<operator_t>::value) {
-      // Claim-first form for operators that come with a bottom-up (owner-exclusive) variant. A thread's four
-      // edges go through the stages together, so the dependent memory round trips of a discovery
-      // (probe -> test-and-set -> degree) overlap across its edges instead of running one discovery after
-      // the other: ncu showed the heavy top-down levels long-scoreboard bound at 19 % issue utilisation with
-      // the per-edge chain (profiles/r01c_merge_path_heavy_push.txt).
-      unsigned word[tile_items], old[tile_items];
+      const unsigned claimed = claim_first(nbr, live, visited);
 #pragma unroll
       for (int i = 0; i < tile_items; ++i)
-        if (live & (1u << i)) word[i] = visited[unsigned(nbr[i]) >> 5];
-#pragma unroll
-      for (int i = 0; i < tile_items; ++i)
-        if ((live & (1u << i)) && ((word[i] >> (unsigned(nbr[i]) & 31u)) & 1u)) live &= ~(1u << i);
-#pragma unroll
-      for (int i = 0; i < tile_items; ++i)
-        if (live & (1u << i)) old[i] = atomicOr(&visited[unsigned(nbr[i]) >> 5], 1u << (unsigned(nbr[i]) & 31u));
-#pragma unroll
-      for (int i = 0; i < tile_items; ++i)
-        if ((live & (1u << i)) && !((old[i] >> (unsigned(nbr[i]) & 31u)) & 1u)) {
+        if (claimed & (1u << i)) {
           const weight_t weight = A.values ? __ldg(A.values + eid[i]) : weight_t(1);
           if (call_pull(op, vertex_t(src[i] + A.source_offset), nbr[i], eid[i], weight)) keep |= 1u << i;
         }
-      if constexpr (count_fresh_edges_in_kernel) {
-        edge_t lo[tile_items], hi[tile_items];
-#pragma unroll
-        for (int i = 0; i < tile_items; ++i)
-          if (keep & (1u << i)) {
-            lo[i] = A.offsets[nbr[i]];
-            hi[i] = A.offsets[nbr[i] + 1];
-          }
-#pragma unroll
-        for (int i = 0; i < tile_items; ++i)
-          if (keep & (1u << i)) fresh_edges += counter_t(hi[i] - lo[i]);
-      }
     } else {
 #pragma unroll
       for (int i = 0; i < tile_items; ++i)
         if (live & (1u << i))
-          if (visit_edge<policy>(A, op, src[i], eid[i], nbr[i], visited, fresh_edges)) keep |= 1u << i;
+          if (visit_edge<policy>(A, op, src[i], eid[i], nbr[i], visited)) keep |= 1u << i;
     }
     if constexpr (has_output)
       b200::cta_append<cta_threads, tile_items>(nbr, keep, output, counters + scratch_t::out_count, capacity,
@@ -213,6 +210,56 @@ __device__ __forceinline__ bool output_fits(counter_t* counters, counter_t capac
   if (worst <= capacity) return true;
   if (blockIdx.x == 0 && threadIdx.x == 0) counters[scratch_t::overflow] = worst;
   return false;
+}
+
+/// Frontier item i (item i is vertex i when the input is the whole graph) and its row: [beg, end), or beg and the
+/// degree when `degree` is set. Past the end of the frontier, and for an invalid id, the vertex is invalid and the
+/// row empty.
+template <bool graph_input, bool degree = false, typename index_t, typename vertex_t, typename edge_t>
+__device__ __forceinline__ void load_row(const edge_t* __restrict__ offsets, const vertex_t* __restrict__ input,
+                                         index_t i, index_t input_size, vertex_t& v, edge_t& beg, edge_t& end) {
+  v = gunrock::numeric_limits<vertex_t>::invalid();
+  beg = 0, end = 0;
+  if (i < input_size) {
+    v = graph_input ? vertex_t(i) : input[i];
+    if (util::limits::is_valid(v)) {
+      beg = offsets[v];
+      end = degree ? offsets[v + 1] - beg : offsets[v + 1];
+    }
+  }
+}
+
+/// Frontier items [first, first + prep_items) of the preparation passes, invalid past the end.
+template <bool graph_input, typename vertex_t>
+__device__ __forceinline__ void load_frontier(const vertex_t* __restrict__ input, std::size_t first,
+                                              std::size_t input_size, vertex_t (&v)[prep_items]) {
+  if constexpr (!graph_input) {
+    // the frontier may be a caller's buffer at any 4-byte offset (a tensor view): 128-bit loads need 16 bytes
+    const bool vector_input = (reinterpret_cast<std::uintptr_t>(input) & 15u) == 0;
+    if (vector_input && first + prep_items <= input_size && prep_items == 4 && sizeof(vertex_t) == 4) {
+      const int4 q = *reinterpret_cast<const int4*>(input + first);  // 128-bit frontier load
+      v[0] = vertex_t(q.x), v[1] = vertex_t(q.y), v[2] = vertex_t(q.z), v[3] = vertex_t(q.w);
+    } else {
+#pragma unroll
+      for (int k = 0; k < prep_items; ++k)
+        v[k] = first + k < input_size ? input[first + k] : gunrock::numeric_limits<vertex_t>::invalid();
+    }
+  } else {
+#pragma unroll
+    for (int k = 0; k < prep_items; ++k)
+      v[k] = first + k < input_size ? vertex_t(first + k) : gunrock::numeric_limits<vertex_t>::invalid();
+  }
+}
+
+/// Writes the neighbour of every lane that keeps it to the output, one atomic per warp. Called by all 32 lanes.
+template <typename vertex_t>
+__device__ __forceinline__ void warp_emit(bool keep, vertex_t nbr, vertex_t* __restrict__ output, counter_t* counters,
+                                          counter_t capacity) {
+  const unsigned votes = __ballot_sync(b200::full_mask, keep);
+  if (votes) {
+    counter_t at = b200::warp_append_slot(keep, counters + scratch_t::out_count);
+    if (keep && at < capacity) output[at] = nbr;
+  }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -258,37 +305,22 @@ __global__ void __launch_bounds__(cta_threads)
   if constexpr (has_output && guard)
     if (!output_fits(counters, capacity)) return;
   if (size_ptr) input_size = std::size_t(*size_ptr);
-  counter_t fresh_edges = 0;
   for (std::size_t base = std::size_t(blockIdx.x) * cta_threads; base < input_size;
        base += std::size_t(gridDim.x) * cta_threads) {
-    const std::size_t i = base + threadIdx.x;
-    vertex_t v = gunrock::numeric_limits<vertex_t>::invalid();
-    edge_t beg = 0, deg = 0;
-    if (i < input_size) {
-      v = graph_input ? vertex_t(i) : input[i];
-      if (util::limits::is_valid(v)) {
-        beg = A.offsets[v];
-        deg = A.offsets[v + 1] - beg;
-      }
-    }
+    vertex_t v;
+    edge_t beg, deg;
+    load_row<graph_input, true>(A.offsets, input, base + threadIdx.x, input_size, v, beg, deg);
     const edge_t trips = b200::warp_max(deg);  // warp-uniform loop so ballots see the whole warp
     for (edge_t k = 0; k < trips; ++k) {
       bool keep = false;
       vertex_t nbr = 0;
       if (k < deg) {
         nbr = __ldg(A.indices + beg + k);
-        keep = visit_edge<policy>(A, op, v, edge_t(beg + k), nbr, visited, fresh_edges);
+        keep = visit_edge<policy>(A, op, v, edge_t(beg + k), nbr, visited);
       }
-      if constexpr (has_output) {
-        const unsigned votes = __ballot_sync(b200::full_mask, keep);
-        if (votes) {
-          counter_t at = b200::warp_append_slot(keep, counters + scratch_t::out_count);
-          if (keep && at < capacity) output[at] = nbr;
-        }
-      }
+      if constexpr (has_output) warp_emit(keep, nbr, output, counters, capacity);
     }
   }
-  flush_fresh_edges<policy>(fresh_edges, counters);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -304,7 +336,6 @@ __global__ void __launch_bounds__(cta_threads)
   const std::size_t count = std::size_t(*size_ptr);
   const unsigned lane = b200::lane_id();
   const std::size_t warps = (std::size_t(gridDim.x) * cta_threads) >> 5;
-  counter_t fresh_edges = 0;
   for (std::size_t item = (std::size_t(blockIdx.x) * cta_threads + threadIdx.x) >> 5; item < count; item += warps) {
     vertex_t v = list[item];
     const edge_t beg = A.offsets[v], end = A.offsets[v + 1];
@@ -314,18 +345,11 @@ __global__ void __launch_bounds__(cta_threads)
       vertex_t nbr = 0;
       if (e < end) {
         nbr = __ldg(A.indices + e);
-        keep = visit_edge<policy>(A, op, v, e, nbr, visited, fresh_edges);
+        keep = visit_edge<policy>(A, op, v, e, nbr, visited);
       }
-      if constexpr (has_output) {
-        const unsigned votes = __ballot_sync(b200::full_mask, keep);
-        if (votes) {
-          counter_t at = b200::warp_append_slot(keep, counters + scratch_t::out_count);
-          if (keep && at < capacity) output[at] = nbr;
-        }
-      }
+      if constexpr (has_output) warp_emit(keep, nbr, output, counters, capacity);
     }
   }
-  flush_fresh_edges<policy>(fresh_edges, counters);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -340,19 +364,11 @@ __global__ void __launch_bounds__(cta_threads)
   __shared__ tile_smem_t<vertex_t, edge_t> sm;
   if constexpr (has_output && guard)
     if (!output_fits(counters, capacity)) return;
-  counter_t fresh_edges = 0;
   for (std::size_t base = std::size_t(blockIdx.x) * cta_threads; base < input_size;
        base += std::size_t(gridDim.x) * cta_threads) {
-    const std::size_t i = base + threadIdx.x;
-    vertex_t v = gunrock::numeric_limits<vertex_t>::invalid();
-    edge_t beg = 0, deg = 0;
-    if (i < input_size) {
-      v = graph_input ? vertex_t(i) : input[i];
-      if (util::limits::is_valid(v)) {
-        beg = A.offsets[v];
-        deg = A.offsets[v + 1] - beg;
-      }
-    }
+    vertex_t v;
+    edge_t beg, deg;
+    load_row<graph_input, true>(A.offsets, input, base + threadIdx.x, input_size, v, beg, deg);
     if (big_list && deg >= edge_t(big_degree)) {  // hub: hand it to the grid-wide kernel
       counter_t at = atomicAdd(counters + scratch_t::big_count, counter_t(1));
       big_list[at] = v;
@@ -369,11 +385,9 @@ __global__ void __launch_bounds__(cta_threads)
     }
     __syncthreads();
     if (n_edges > 0)
-      expand_tile<has_output, policy>(A, op, sm, int(n_seg), n_edges, output, counters, capacity, visited,
-                                      fresh_edges);
+      expand_tile<has_output, policy>(A, op, sm, int(n_seg), n_edges, output, counters, capacity, visited);
     __syncthreads();
   }
-  flush_fresh_edges<policy>(fresh_edges, counters);
 }
 
 /// Grid-wide expansion of the deferred hubs: every CTA strides the 1024-edge tiles of each listed vertex.
@@ -386,7 +400,6 @@ __global__ void __launch_bounds__(cta_threads)
   if constexpr (has_output)
     if (!output_fits(counters, capacity)) return;
   const std::size_t count = std::size_t(*size_ptr);
-  counter_t fresh_edges = 0;
   for (std::size_t item = 0; item < count; ++item) {
     const vertex_t v = big_list[item];
     const edge_t beg = A.offsets[v], deg = A.offsets[v + 1] - beg;
@@ -399,11 +412,10 @@ __global__ void __launch_bounds__(cta_threads)
       __syncthreads();
       const edge_t left = deg - t0;
       expand_tile<has_output, policy>(A, op, sm, 1, left < edge_t(tile_edges) ? left : edge_t(tile_edges), output,
-                                      counters, capacity, visited, fresh_edges);
+                                      counters, capacity, visited);
       __syncthreads();
     }
   }
-  flush_fresh_edges<policy>(fresh_edges, counters);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -421,8 +433,6 @@ __global__ void __launch_bounds__(cta_threads)
   __shared__ unsigned long long prefix[2];
   __shared__ int s_tile;
   const int n_tiles = int((input_size + per_tile - 1) / per_tile);
-  // the frontier may be a caller's buffer at any 4-byte offset (a tensor view): 128-bit loads need 16 bytes
-  const bool vector_input = (reinterpret_cast<std::uintptr_t>(input) & 15u) == 0;
   for (;;) {
     if (threadIdx.x == 0) s_tile = int(atomicAdd(counters + scratch_t::ticket, counter_t(1)));
     __syncthreads();
@@ -431,20 +441,7 @@ __global__ void __launch_bounds__(cta_threads)
     const std::size_t first = std::size_t(tile) * per_tile + std::size_t(threadIdx.x) * prep_items;
     vertex_t v[prep_items];
     edge_t beg[prep_items], deg[prep_items];
-    if constexpr (!graph_input) {
-      if (vector_input && first + prep_items <= input_size && prep_items == 4 && sizeof(vertex_t) == 4) {
-        const int4 q = *reinterpret_cast<const int4*>(input + first);  // 128-bit frontier load
-        v[0] = vertex_t(q.x), v[1] = vertex_t(q.y), v[2] = vertex_t(q.z), v[3] = vertex_t(q.w);
-      } else {
-#pragma unroll
-        for (int k = 0; k < prep_items; ++k)
-          v[k] = first + k < input_size ? input[first + k] : gunrock::numeric_limits<vertex_t>::invalid();
-      }
-    } else {
-#pragma unroll
-      for (int k = 0; k < prep_items; ++k)
-        v[k] = first + k < input_size ? vertex_t(first + k) : gunrock::numeric_limits<vertex_t>::invalid();
-    }
+    load_frontier<graph_input>(input, first, input_size, v);
     unsigned my_items = 0;
     unsigned long long my_edges = 0;
 #pragma unroll
@@ -505,7 +502,6 @@ __global__ void __launch_bounds__(cta_threads)
     if (!output_fits(counters, capacity)) return;
   const long long total = (long long)counters[scratch_t::work_total];
   const long long n_items = (long long)counters[scratch_t::items];
-  counter_t fresh_edges = 0;
   // Each CTA takes a CONTIGUOUS run of 1024-edge slices, so only its first slice needs the binary search on
   // the scanned offsets (17 dependent L2 round trips at |F| = 120 K while 254 threads wait); every following
   // slice starts in the segment the previous one ended in and its last segment is found from shared memory.
@@ -555,8 +551,7 @@ __global__ void __launch_bounds__(cta_threads)
       n_seg = int(total_seg);
     }
     __syncthreads();
-    expand_tile<has_output, policy>(A, op, sm, n_seg, edge_t(g1 - g0), output, counters, capacity, visited,
-                                    fresh_edges);
+    expand_tile<has_output, policy>(A, op, sm, n_seg, edge_t(g1 - g0), output, counters, capacity, visited);
     // next slice starts in the last segment of this one if that segment continues past g1, else in the next
     {
       const long long last = j0 + n_seg - 1;
@@ -565,7 +560,6 @@ __global__ void __launch_bounds__(cta_threads)
     }
     __syncthreads();
   }
-  flush_fresh_edges<policy>(fresh_edges, counters);
 }
 
 // merge_path for small frontiers (nf <= tile_edges items): ONE launch. Every CTA redundantly builds the whole
@@ -587,15 +581,7 @@ __global__ void __launch_bounds__(cta_threads)
 #pragma unroll
   for (int k = 0; k < tile_items; ++k) {
     const int i = int(threadIdx.x) * tile_items + k;  // blocked order keeps the table in frontier order
-    v[k] = gunrock::numeric_limits<vertex_t>::invalid();
-    beg[k] = deg[k] = 0;
-    if (i < input_size) {
-      v[k] = graph_input ? vertex_t(i) : input[i];
-      if (util::limits::is_valid(v[k])) {
-        beg[k] = A.offsets[v[k]];
-        deg[k] = A.offsets[v[k] + 1] - beg[k];
-      }
-    }
+    load_row<graph_input, true>(A.offsets, input, i, input_size, v[k], beg[k], deg[k]);
     my_items += deg[k] > 0;
     my_edges += deg[k];
   }
@@ -620,13 +606,11 @@ __global__ void __launch_bounds__(cta_threads)
       return;
     }
   }
-  counter_t fresh_edges = 0;
   for (edge_t g0 = edge_t(blockIdx.x) * tile_edges; g0 < total; g0 += edge_t(gridDim.x) * tile_edges) {
     const edge_t left = total - g0;
     expand_tile<has_output, policy>(A, op, sm, int(n_seg), left < edge_t(tile_edges) ? left : edge_t(tile_edges),
-                                    output, counters, capacity, visited, fresh_edges, g0);
+                                    output, counters, capacity, visited, g0);
   }
-  flush_fresh_edges<policy>(fresh_edges, counters);
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -125,7 +125,7 @@ template <visit_t policy, int QPL, typename vertex_t, typename edge_t, typename 
 __device__ __forceinline__ unsigned visit_items(const graph::adjacency_t<vertex_t, edge_t, weight_t>& A, operator_t& op,
                                                 const vertex_t (&nbr)[QPL * 4], unsigned live,
                                                 const vertex_t (&src)[QPL], const edge_t (&e0)[QPL],
-                                                unsigned* __restrict__ visited, counter_t& fresh_edges) {
+                                                unsigned* __restrict__ visited) {
   constexpr int N = QPL * 4;
   unsigned keep = 0;
   weight_t wt[N];
@@ -144,43 +144,18 @@ __device__ __forceinline__ unsigned visit_items(const graph::adjacency_t<vertex_
   };
 
   if constexpr (policy == visit_t::test_and_set && has_pull_operator<operator_t>::value) {
-    // claim-first: all probes of the lane's edges are in flight together, then the (few) test-and-sets, then the
-    // owner-exclusive form of the operator on the claimed neighbours
-    unsigned word[N];
-#pragma unroll
-    for (int i = 0; i < N; ++i)
-      if (live & (1u << i)) word[i] = visited[unsigned(nbr[i]) >> 5];
-#pragma unroll
-    for (int i = 0; i < N; ++i)
-      if ((live & (1u << i)) && ((word[i] >> (unsigned(nbr[i]) & 31u)) & 1u)) live &= ~(1u << i);
-    unsigned claimed = 0;
-#pragma unroll
-    for (int i = 0; i < N; ++i)
-      if (live & (1u << i)) {
-        const unsigned bit = 1u << (unsigned(nbr[i]) & 31u);
-        if (!(atomicOr(&visited[unsigned(nbr[i]) >> 5], bit) & bit)) claimed |= 1u << i;
-      }
+    const unsigned claimed = claim_first(nbr, live, visited);
     if (claimed) {
       load_weights(claimed);
 #pragma unroll
       for (int i = 0; i < N; ++i)
-        if (claimed & (1u << i)) {
+        if (claimed & (1u << i))
           if (call_pull(op, vertex_t(src[i >> 2] + A.source_offset), nbr[i], edge_t(e0[i >> 2] + (i & 3)), wt[i]))
             keep |= 1u << i;
-          if constexpr (count_fresh_edges_in_kernel)
-            fresh_edges += counter_t(A.offsets[nbr[i] + 1] - A.offsets[nbr[i]]);
-        }
     }
   } else {
-    if constexpr (policy == visit_t::test_and_set) {
-      unsigned word[N];
-#pragma unroll
-      for (int i = 0; i < N; ++i)
-        if (live & (1u << i)) word[i] = visited[unsigned(nbr[i]) >> 5];
-#pragma unroll
-      for (int i = 0; i < N; ++i)
-        if ((live & (1u << i)) && ((word[i] >> (unsigned(nbr[i]) & 31u)) & 1u)) live &= ~(1u << i);
-    }
+    // the whole batch is probed before the operator runs on any edge
+    if constexpr (policy == visit_t::test_and_set) live = drop_visited(nbr, live, visited);
     load_weights(live);
 #pragma unroll
     for (int i = 0; i < N; ++i)
@@ -188,23 +163,7 @@ __device__ __forceinline__ unsigned visit_items(const graph::adjacency_t<vertex_
         vertex_t s = src[i >> 2] + A.source_offset, d = nbr[i];  // 1-D partition: global source id
         edge_t e = edge_t(e0[i >> 2] + (i & 3));
         weight_t w = wt[i];
-        bool k = op(s, d, e, w);  // lvalues, exactly once per live edge
-        if constexpr (policy == visit_t::test_and_set) {
-          if (k) {
-            const unsigned bit = 1u << (unsigned(d) & 31u);
-            k = !(atomicOr(&visited[unsigned(d) >> 5], bit) & bit);
-            if constexpr (count_fresh_edges_in_kernel)
-              if (k) fresh_edges += counter_t(A.offsets[d + 1] - A.offsets[d]);
-          }
-        }
-        if constexpr (policy == visit_t::unique_output) {
-          if (k) {
-            const unsigned bit = 1u << (unsigned(d) & 31u);
-            unsigned* word = &visited[unsigned(d) >> 5];
-            k = !(*word & bit) && !(atomicOr(word, bit) & bit);
-          }
-        }
-        if (k) keep |= 1u << i;
+        if (admit<policy>(visited, unsigned(d), op(s, d, e, w))) keep |= 1u << i;  // lvalues, once per live edge
       }
   }
   return keep;
@@ -244,7 +203,7 @@ __device__ __forceinline__ void expand_round(const graph::adjacency_t<vertex_t, 
                                              const edge_t* end, const vertex_t* src_of, int n_seg, edge_t pos0,
                                              int n_quads, vertex_t* sbuf, unsigned& staged,
                                              vertex_t* __restrict__ output, counter_t* counters, counter_t capacity,
-                                             unsigned* __restrict__ visited, counter_t& fresh_edges) {
+                                             unsigned* __restrict__ visited) {
   const int lane = int(b200::lane_id());
   vertex_t src[quads_per_lane];
   edge_t e0[quads_per_lane], lo[quads_per_lane], hi[quads_per_lane];
@@ -272,7 +231,7 @@ __device__ __forceinline__ void expand_round(const graph::adjacency_t<vertex_t, 
     for (int i = 0; i < 4; ++i) nbr[4 * q + i] = c[i];
   }
   const unsigned live = live_mask<quads_per_lane>(have, e0, lo, hi);
-  const unsigned keep = visit_items<policy, quads_per_lane>(A, op, nbr, live, src, e0, visited, fresh_edges);
+  const unsigned keep = visit_items<policy, quads_per_lane>(A, op, nbr, live, src, e0, visited);
   if constexpr (has_output)
     stage_append<CAP>(nbr, keep, sbuf, staged, output, counters + scratch_t::out_count, capacity);
 }
@@ -293,8 +252,6 @@ __global__ void __launch_bounds__(cta_threads)
   __shared__ unsigned long long prefix[2];
   __shared__ int s_tile;
   const int n_tiles = int((input_size + per_tile - 1) / per_tile);
-  // the frontier may be a caller's buffer at any 4-byte offset (a tensor view): 128-bit loads need 16 bytes
-  const bool vector_input = (reinterpret_cast<std::uintptr_t>(input) & 15u) == 0;
   for (;;) {
     if (threadIdx.x == 0) s_tile = int(atomicAdd(counters + scratch_t::ticket, counter_t(1)));
     __syncthreads();
@@ -303,20 +260,7 @@ __global__ void __launch_bounds__(cta_threads)
     const std::size_t first = std::size_t(tile) * per_tile + std::size_t(threadIdx.x) * prep_items;
     vertex_t v[prep_items];
     edge_t beg[prep_items], end[prep_items];
-    if constexpr (!graph_input) {
-      if (vector_input && first + prep_items <= input_size && prep_items == 4 && sizeof(vertex_t) == 4) {
-        const int4 q = *reinterpret_cast<const int4*>(input + first);  // 128-bit frontier load
-        v[0] = vertex_t(q.x), v[1] = vertex_t(q.y), v[2] = vertex_t(q.z), v[3] = vertex_t(q.w);
-      } else {
-#pragma unroll
-        for (int k = 0; k < prep_items; ++k)
-          v[k] = first + k < input_size ? input[first + k] : gunrock::numeric_limits<vertex_t>::invalid();
-      }
-    } else {
-#pragma unroll
-      for (int k = 0; k < prep_items; ++k)
-        v[k] = first + k < input_size ? vertex_t(first + k) : gunrock::numeric_limits<vertex_t>::invalid();
-    }
+    load_frontier<graph_input>(input, first, input_size, v);
     unsigned my_items = 0;
     unsigned long long my_quads = 0, my_edges = 0;
     unsigned long long nq[prep_items];
@@ -399,7 +343,6 @@ __global__ void __launch_bounds__(cta_threads, 4)
   auto& T = tables[warp];
   vertex_t* sbuf = stages[has_output ? warp : 0].buf;
   unsigned staged = 0;
-  counter_t fresh_edges = 0;
 
   const long long n_rounds = (total + round_quads - 1) / round_quads;
   const long long n_warps = (long long)gridDim.x * quad_warps;
@@ -447,8 +390,7 @@ __global__ void __launch_bounds__(cta_threads, 4)
       }
       __syncwarp();
       expand_round<has_output, policy, stage_cap>(A, op, T.rel, T.qoff, T.beg, T.end, T.src, n_seg, edge_t(0),
-                                                  int(rend - r), sbuf, staged, output, counters, capacity, visited,
-                                                  fresh_edges);
+                                                  int(rend - r), sbuf, staged, output, counters, capacity, visited);
       {  // the next round starts in this round's last list when that list continues past rend
         const int last = n_seg - 1;
         const long long last_stop = r - (long long)T.qoff[last] + (long long)((T.end[last] - 1) >> 2) + 1;
@@ -458,7 +400,6 @@ __global__ void __launch_bounds__(cta_threads, 4)
     }
   }
   if constexpr (has_output) stage_flush(sbuf, staged, output, counters + scratch_t::out_count, capacity);
-  flush_fresh_edges<policy>(fresh_edges, counters);
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -523,23 +464,15 @@ __global__ void __launch_bounds__(cta_threads, 4)
   const unsigned warp = b200::warp_id();
   vertex_t* sbuf = stages[has_output ? warp : 0].buf;
   unsigned staged = 0;
-  counter_t fresh_edges = 0;
   const std::size_t n_tiles = (input_size + cta_threads - 1) / cta_threads;
   for (;;) {
     if (threadIdx.x == 0) T.ticket = int(atomicAdd(counters + scratch_t::ticket, counter_t(1)));
     __syncthreads();
     const std::size_t tile = std::size_t(T.ticket);
     if (tile >= n_tiles) break;
-    const std::size_t i = tile * cta_threads + threadIdx.x;
-    vertex_t v[1] = {gunrock::numeric_limits<vertex_t>::invalid()};
-    edge_t beg[1] = {0}, end[1] = {0};
-    if (i < input_size) {
-      v[0] = graph_input ? vertex_t(i) : input[i];
-      if (util::limits::is_valid(v[0])) {
-        beg[0] = A.offsets[v[0]];
-        end[0] = A.offsets[v[0] + 1];
-      }
-    }
+    vertex_t v[1];
+    edge_t beg[1], end[1];
+    load_row<graph_input>(A.offsets, input, tile * cta_threads + threadIdx.x, input_size, v[0], beg[0], end[0]);
     if (big_list && end[0] - beg[0] >= edge_t(big_degree)) {  // hub: hand it to the grid-wide kernel
       const counter_t at = atomicAdd(counters + scratch_t::big_count, counter_t(1));
       big_list[at] = v[0];
@@ -554,12 +487,11 @@ __global__ void __launch_bounds__(cta_threads, 4)
       const edge_t left = n_quads - pos0;
       expand_round<has_output, policy, stage_cap>(A, op, T.rel, T.qoff, T.beg, T.end, T.src, int(n_seg), pos0,
                                                   int(left < edge_t(round_quads) ? left : edge_t(round_quads)), sbuf,
-                                                  staged, output, counters, capacity, visited, fresh_edges);
+                                                  staged, output, counters, capacity, visited);
     }
     __syncthreads();  // table and ticket reuse
   }
   if constexpr (has_output) stage_flush(sbuf, staged, output, counters + scratch_t::out_count, capacity);
-  flush_fresh_edges<policy>(fresh_edges, counters);
 }
 
 // merge_path for small frontiers (nf <= small_items): ONE launch. Every CTA builds the whole table in shared
@@ -582,15 +514,7 @@ __global__ void __launch_bounds__(cta_threads, 4)
 #pragma unroll
   for (int k = 0; k < per_thread; ++k) {
     const int i = int(threadIdx.x) * per_thread + k;  // blocked order keeps the table in frontier order
-    v[k] = gunrock::numeric_limits<vertex_t>::invalid();
-    beg[k] = end[k] = 0;
-    if (i < input_size) {
-      v[k] = graph_input ? vertex_t(i) : input[i];
-      if (util::limits::is_valid(v[k])) {
-        beg[k] = A.offsets[v[k]];
-        end[k] = A.offsets[v[k] + 1];
-      }
-    }
+    load_row<graph_input>(A.offsets, input, i, input_size, v[k], beg[k], end[k]);
     my_edges += (unsigned long long)(end[k] - beg[k]);
   }
   my_edges = b200::warp_sum(my_edges);
@@ -609,7 +533,6 @@ __global__ void __launch_bounds__(cta_threads, 4)
   const unsigned warp = b200::warp_id();
   vertex_t* sbuf = stages[has_output ? warp : 0].buf;
   unsigned staged = 0;
-  counter_t fresh_edges = 0;
   const edge_t rounds = (n_quads + round_quads - 1) / round_quads;
   for (edge_t round = edge_t(blockIdx.x) * quad_warps + edge_t(warp); round < rounds;
        round += edge_t(gridDim.x) * quad_warps) {
@@ -617,10 +540,9 @@ __global__ void __launch_bounds__(cta_threads, 4)
     const edge_t left = n_quads - pos0;
     expand_round<has_output, policy, stage_cap>(A, op, T.rel, T.qoff, T.beg, T.end, T.src, int(n_seg), pos0,
                                                 int(left < edge_t(round_quads) ? left : edge_t(round_quads)), sbuf,
-                                                staged, output, counters, capacity, visited, fresh_edges);
+                                                staged, output, counters, capacity, visited);
   }
   if constexpr (has_output) stage_flush(sbuf, staged, output, counters + scratch_t::out_count, capacity);
-  flush_fresh_edges<policy>(fresh_edges, counters);
 }
 
 // warp_mapped over quads: one warp per list item (bucketing's medium bin), lanes stride the list's quads.
@@ -637,7 +559,6 @@ __global__ void __launch_bounds__(cta_threads, 4)
   const std::size_t warps = std::size_t(gridDim.x) * quad_warps;
   vertex_t* sbuf = stages[has_output ? warp : 0].buf;
   unsigned staged = 0;
-  counter_t fresh_edges = 0;
   for (std::size_t item = std::size_t(blockIdx.x) * quad_warps + warp; item < count; item += warps) {
     const vertex_t v = list[item];
     const edge_t beg = A.offsets[v], end = A.offsets[v + 1];
@@ -662,13 +583,12 @@ __global__ void __launch_bounds__(cta_threads, 4)
         for (int i = 0; i < 4; ++i) nbr[4 * q + i] = c[i];
       }
       const unsigned live = live_mask<quads_per_lane>(have, e0, lo, hi);
-      const unsigned keep = visit_items<policy, quads_per_lane>(A, op, nbr, live, src, e0, visited, fresh_edges);
+      const unsigned keep = visit_items<policy, quads_per_lane>(A, op, nbr, live, src, e0, visited);
       if constexpr (has_output)
         stage_append<stage_cap>(nbr, keep, sbuf, staged, output, counters + scratch_t::out_count, capacity);
     }
   }
   if constexpr (has_output) stage_flush(sbuf, staged, output, counters + scratch_t::out_count, capacity);
-  flush_fresh_edges<policy>(fresh_edges, counters);
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -740,7 +660,6 @@ __global__ void __launch_bounds__(cta_threads, 4)
   const unsigned warp = b200::warp_id();
   vertex_t* sbuf = stages[has_output ? warp : 0].buf;
   unsigned staged = 0;
-  counter_t fresh_edges = 0;
   if (threadIdx.x == 0) {
     mbarrier_init(&s_bar[0], 1);
     mbarrier_init(&s_bar[1], 1);
@@ -838,7 +757,7 @@ __global__ void __launch_bounds__(cta_threads, 4)
         for (int i = 0; i < 4; ++i) nbr[4 * q + i] = c[i];
       }
       const unsigned live = live_mask<quads_per_lane>(have, e0, lo, hi);
-      const unsigned keep = visit_items<policy, quads_per_lane>(A, op, nbr, live, src, e0, visited, fresh_edges);
+      const unsigned keep = visit_items<policy, quads_per_lane>(A, op, nbr, live, src, e0, visited);
       if constexpr (has_output)
         stage_append<stage_cap>(nbr, keep, sbuf, staged, output, counters + scratch_t::out_count, capacity);
       __syncthreads();  // everyone is done with s_col[stage] before it is refilled two tiles from now
@@ -850,7 +769,6 @@ __global__ void __launch_bounds__(cta_threads, 4)
     __syncthreads();  // batch tables are rewritten by the next iteration
   }
   if constexpr (has_output) stage_flush(sbuf, staged, output, counters + scratch_t::out_count, capacity);
-  flush_fresh_edges<policy>(fresh_edges, counters);
 }
 
 }  // namespace kernels
