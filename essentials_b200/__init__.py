@@ -368,7 +368,8 @@ def pagerank(ctx: Context, g: Graph, alpha: float = 0.85, tol: float = 1e-6, max
     per element — this is the parity path. `pull=False` is the reference's formulation, an advance that scatters
     `atomic::add` over the out-edges with balancer `lb`; float additions then arrive in whatever order the hardware
     schedules them, so individual ranks can differ by up to ~1e-4 relative from run to run (1e-6 in L1), exactly as
-    the reference's GPU PageRank does. Without an in-edge view the default is the scatter."""
+    the reference's GPU PageRank does. Without an in-edge view the default is the scatter. The gather raises
+    :class:`EssentialsError` when only one of the CSR and the CSC carries edge weights."""
     import torch
     p = _out(g.n, torch.float32, g) if out is None else out
     info = RunInfo()

@@ -150,7 +150,8 @@ ESS_API int ess_sssp_delta(ess_context_t ctx, ess_graph_t g, int32_t source, flo
                            ess_run_info* info);
 
 /* gunrock::pr::run — include/gunrock/algorithms/pr.hxx:183-216 (alpha 0.85, tol 1e-6 in examples/algorithms/pr/pr.cu:55-56).
- * pull != 0 gathers over the CSC view instead of scattering with atomics. */
+ * pull != 0 gathers over the CSC view instead of scattering with atomics; it fails when only one of the CSR and
+ * CSC views carries edge weights. */
 ESS_API int ess_pagerank(ess_context_t ctx, ess_graph_t g, float alpha, float tol, int max_iterations, float* d_p, int lb,
                  int pull, ess_run_info* info);
 

@@ -221,6 +221,10 @@ struct problem_t : gunrock::problem_t<graph_t> {
     auto* ctx = this->get_single_context();
     auto g = this->get_graph();
     const auto A = graph::adjacency_of<true>(g);
+    // iweights sums the CSR weights and the gather multiplies by the CSC ones: with weights on only one view the
+    // ranks would be silently wrong, so refuse the graph.
+    error::throw_if_exception(A.m > 0 && (A.values == nullptr) != (graph::adjacency_of<false>(g).values == nullptr),
+                              "pr: pull needs edge weights on both the CSR and the CSC view, or on neither");
     const std::size_t n = std::size_t(A.n);
     contrib.resize(n);
     short_rows.resize(n);
