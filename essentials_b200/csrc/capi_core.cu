@@ -83,20 +83,8 @@ int ess_context_synchronize(ess_context_t ctx) {
 int ess_tune(const char* knob, int value) {
   ESS_TRY
   const std::string k = knob ? knob : "";
-  if (k == "near_far_ctas") {
-    gunrock::operators::advance::near_far_ctas_per_sm() = value < 1 ? 1 : value;
-    return 0;
-  }
   if (k == "advance_engine") {  // 1 = quad engine (128-bit loads, warp-autonomous rounds), 0 = round-1 scalar kernels
     gunrock::operators::advance::kernels::advance_engine() = value;
-    return 0;
-  }
-  if (k == "pull_engine") {  // 1 = pull_chunk_kernel, 0 = pull_step_kernel
-    gunrock::operators::advance::kernels::pull_engine() = value;
-    return 0;
-  }
-  if (k == "near_far_cluster") {  // 1 = small levels of execute_near_far run in one thread-block cluster
-    gunrock::operators::advance::near_far_cluster_enabled() = value;
     return 0;
   }
   if (k == "pull_hints") {

@@ -101,15 +101,11 @@ inline int fail_pull_via_step() {
   return ess::fail("ess_bfs_partition_step: bottom-up levels go through ess_bfs_partition_pull");
 }
 
-/// Copies (out_count, aux2) of the operator counter block into the caller's two int64 and re-zeroes the block.
-static __global__ void export_counts_kernel(b200::counter_t* counters, b200::counter_t* counts, bool has_edges) {
-  // has_edges: aux2 holds Σdeg of the vertices found (pull_step_kernel); pull_chunk_kernel does not read row bounds
-  // of the vertices it adopts, so Beamer's m_f is simply not updated on bottom-up levels (only the top-down rule
-  // uses it, and absorb_kernel supplies it there)
-  if (threadIdx.x == 0) {
-    counts[0] += counters[scratch_t::out_count];
-    if (has_edges) counts[1] += counters[scratch_t::aux2];
-  }
+/// Adds out_count of the operator counter block to the caller's counts[0] and re-zeroes the block. counts[1] (Σdeg
+/// of the vertices found) is left alone: the pull kernel does not read row bounds of the vertices it adopts, and only
+/// the top-down rule uses Beamer's m_f, which absorb_kernel supplies there.
+static __global__ void export_counts_kernel(b200::counter_t* counters, b200::counter_t* counts) {
+  if (threadIdx.x == 0) counts[0] += counters[scratch_t::out_count];
   if (threadIdx.x < scratch_t::n_slots) counters[threadIdx.x] = 0;
 }
 
@@ -131,17 +127,12 @@ int partition_pull(ess_context_t ctx, graph_t& G, int64_t row_begin, int32_t lev
   scratch.zero(stream);
   c->profiler().begin(gcuda::profiler_t::pull_step, stream);
   namespace k = operators::advance::kernels;
-  const bool chunked = k::pull_engine() != 0;
-  if (chunked) {  // same kernel as the single-GPU bottom-up level: rows, visited and next words are the owned range
-    auto kernel = k::pull_chunk_kernel<int32_t, edge_t, float, decltype(adopt)>;
-    const std::size_t chunks = ((std::size_t(A.n) + 31) / 32 + k::pull_chunk_words - 1) / k::pull_chunk_words;
-    kernel<<<gcuda::full_grid(*c, kernel, (chunks + 7) / 8), 256, 0, stream>>>(
-        A, adopt, d_frontier_bits, d_next_slice, d_visited_bits + (row_begin >> 5), scratch.d);
-  } else {
-    k::pull_step_kernel<<<gcuda::persistent_grid(*c, (std::size_t(A.n) + 255) / 256, 6), 256, 0, stream>>>(
-        A, adopt, d_frontier_bits, d_next_slice, d_visited_bits + (row_begin >> 5), scratch.d);
-  }
-  export_counts_kernel<<<1, 32, 0, stream>>>(scratch.d, reinterpret_cast<b200::counter_t*>(d_counts), !chunked);
+  // same kernel as the single-GPU bottom-up level: rows, visited and next words are the owned range
+  auto kernel = k::pull_chunk_kernel<int32_t, edge_t, float, decltype(adopt)>;
+  const std::size_t chunks = ((std::size_t(A.n) + 31) / 32 + k::pull_chunk_words - 1) / k::pull_chunk_words;
+  kernel<<<gcuda::full_grid(*c, kernel, (chunks + 7) / 8), 256, 0, stream>>>(
+      A, adopt, d_frontier_bits, d_next_slice, d_visited_bits + (row_begin >> 5), scratch.d);
+  export_counts_kernel<<<1, 32, 0, stream>>>(scratch.d, reinterpret_cast<b200::counter_t*>(d_counts));
   c->profiler().end(stream, 2);
   scratch.clean = true;  // export_counts_kernel re-zeroed the block
   error::check_last("partition pull");

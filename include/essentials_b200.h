@@ -239,7 +239,8 @@ ESS_API int ess_bfs_partition_step(ess_context_t ctx, ess_graph_t g, int64_t row
                                    int64_t frontier_count);
  /* ess_bfs_partition_pull, one bottom-up level on the owned rows with the single-GPU pull kernel: every owned
  * vertex outside d_visited_bits that has an in-neighbour in d_frontier_bits gets depth = level, joins visited
- * and d_next_slice (owned words); d_counts[0] += |fresh|, d_counts[1] += sum of their degrees. */
+ * and d_next_slice (owned words); d_counts[0] += |fresh|. d_counts[1] is not changed: the kernel reads no row
+ * bounds of the vertices it adopts, so the sum of their degrees is not known. */
 ESS_API int ess_bfs_partition_pull(ess_context_t ctx, ess_graph_t g, int64_t row_begin, int32_t level,
                                    const uint32_t* d_frontier_bits, uint32_t* d_visited_bits,
                                    uint32_t* d_next_slice, int32_t* d_depth_local, int64_t* d_counts);

@@ -448,26 +448,20 @@ void optimized(graph_t& G, enactor_type* E, operator_t op, gcuda::standard_conte
     auto& nxt = D.dense[D.dense_selector ^ 1];
     scratch.zero(stream);
     prof.begin(profiler_t::pull_step, stream);
-    const bool chunked = kernels::pull_engine() != 0;
-    if (chunked) {
-      const std::size_t chunks = ((std::size_t(n) + 31) / 32 + kernels::pull_chunk_words - 1) / kernels::pull_chunk_words;
-      auto kernel = kernels::pull_chunk_kernel<vertex_t, edge_t, typename graph_t::weight_type, operator_t>;
-      kernel<<<gcuda::full_grid(ctx, kernel, (chunks + 7) / 8), 256, 0, stream>>>(in_adj, op, cur.data(), nxt.data(),
-                                                                                  D.visited.data(), scratch.d);
-    } else {
-      kernels::pull_step_kernel<<<gcuda::persistent_grid(ctx, (std::size_t(n) + 255) / 256, 6), 256, 0, stream>>>(
-          in_adj, op, cur.data(), nxt.data(), D.visited.data(), scratch.d);
-    }
+    const std::size_t chunks = ((std::size_t(n) + 31) / 32 + kernels::pull_chunk_words - 1) / kernels::pull_chunk_words;
+    auto kernel = kernels::pull_chunk_kernel<vertex_t, edge_t, typename graph_t::weight_type, operator_t>;
+    kernel<<<gcuda::full_grid(ctx, kernel, (chunks + 7) / 8), 256, 0, stream>>>(in_adj, op, cur.data(), nxt.data(),
+                                                                                D.visited.data(), scratch.d);
     prof.end(stream);
     error::check_last("pull step");
     scratch.fetch(stream);
     next_vertices = (long long)scratch.h[scratch_t::out_count];
-    // the chunked kernel does not read row bounds of the vertices it adopts, so Σdeg of the next frontier is
+    // the pull kernel does not read row bounds of the vertices it adopts, so Σdeg of the next frontier is
     // unknown while pulling; it is recomputed from the sparse list on the way back to top-down (below)
-    next_edges = chunked ? 0 : (long long)scratch.h[scratch_t::aux2];
+    next_edges = 0;
     D.pull_vertices_scanned += (long long)scratch.h[scratch_t::aux0];
     D.pull_edges_inspected += (long long)scratch.h[scratch_t::aux1];
-    if (chunked) D.pull_hint_misses += (long long)scratch.h[scratch_t::aux2];
+    D.pull_hint_misses += (long long)scratch.h[scratch_t::aux2];
     D.pull_vertices_found += next_vertices;
     D.dense_selector ^= 1;
     D.dense[D.dense_selector].set_number_of_elements(std::size_t(next_vertices));

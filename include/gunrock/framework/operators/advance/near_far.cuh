@@ -51,27 +51,18 @@ struct near_far_state_t {
   int levels;    ///< near levels executed
   int splits;    ///< far-pile splits executed
   int overflow;  ///< a queue ran out of capacity (impossible with capacity n thanks to the stamps; checked anyway)
-  int level;     ///< next near level to run (lets the grid-wide and the cluster kernel hand the run to each other)
-  int exit_reason;  ///< why the kernel returned: see near_far_exit_t
-};
-
-/// Why a near-far kernel returned to the host.
-enum near_far_exit_t : int {
-  near_far_done = 0,       ///< near queue and far pile empty (or max_levels reached)
-  near_far_grew = 1,       ///< cluster kernel: the work outgrew one cluster; continue with the grid-wide kernel
-  near_far_shrank = 2      ///< grid-wide kernel: the near queue fits one cluster again
 };
 
 constexpr unsigned near_far_inf_bits = 0x7f800000u;
 
 /**
- * @brief One near level, shared by the grid-wide and the cluster kernel: every lane takes one vertex of the level's
- * queue; its edges are relaxed 4 per batch so that the column/weight loads, the operators (atomics) and the routing
+ * @brief One near level of near_far_kernel: every lane takes one vertex of the level's queue; its edges are relaxed
+ * 4 per batch so that the column/weight loads, the operators (atomics) and the routing
  * (priority loads, stamp / flag exchanges) of a batch are in flight together — the edge-at-a-time loop this
  * replaces paid one full dependent chain of L2 round trips PER EDGE, most of a level's 13-15 us on the grid. A
  * neighbour the operator improved joins the next near queue (priority < threshold, once per level: stamp) or the
- * far pile (once: flag); the warp claims its slots with ONE atomic per queue and batch. `out_count` / `far_count`
- * may live in global or in distributed shared memory. Called by all threads of the kernel.
+ * far pile (once: flag); the warp claims its slots with ONE atomic per queue and batch. Called by all threads of the
+ * kernel.
  */
 template <typename vertex_t, typename edge_t, typename weight_t, typename operator_t, typename priority_t>
 __device__ __forceinline__ void near_far_expand_level(
@@ -82,7 +73,7 @@ __device__ __forceinline__ void near_far_expand_level(
     unsigned long long threads, unsigned long long& my_relax, bool& overflowed) {
   const unsigned lane = b200::lane_id();
   // Routes up to 4 improved neighbours per lane: priorities, stamps and flags of the batch are in flight
-  // together, and the whole warp claims its queue slots with ONE distributed-shared-memory atomic per queue.
+  // together, and the whole warp claims its queue slots with ONE atomic per queue.
   auto route4 = [&](const bool (&improved)[4], const vertex_t (&u)[4]) {  // called by all 32 lanes
     float pri[4];
     int previous[4];
@@ -237,23 +228,16 @@ __device__ __forceinline__ void near_far_expand_level(
 }
 
 /**
- * @brief The whole traversal, shared by the two kernels below; `sync()` is the device-wide (cooperative grid) or the
- * cluster-wide (hardware barrier.cluster) barrier — both order global memory among the threads they join.
- * shrink_limit > 0: return near_far_shrank as soon as a near level holds at most that many vertices (grid-wide
- * kernel: the host continues in the cluster kernel, whose barrier is several times cheaper). grow_limit > 0: return
- * near_far_grew when a near level exceeds it or the far pile exceeds 64 x it (cluster kernel -> grid-wide kernel).
- * Queue lengths, threshold and selectors live in `state` (global memory, L2): a first version of the cluster kernel
- * kept them in the leader CTA's shared memory and appended through distributed-shared-memory atomics — ~600 remote
- * atomics per level serialised on one SM's shared-memory port and cost more than the barrier saved.
+ * @brief The whole traversal (see file comment): one cooperative launch of 256-thread CTAs, one grid barrier per
+ * level. Queue lengths, threshold and selectors live in `state` (global memory, L2). A thread-block-cluster form, whose
+ * barrier is cheaper, was measured slower on the 4900 x 4900 grid (DESIGN.md §3.3).
  */
-template <typename vertex_t, typename edge_t, typename weight_t, typename operator_t, typename priority_t,
-          typename sync_t>
-__device__ __forceinline__ void near_far_run(const graph::adjacency_t<vertex_t, edge_t, weight_t>& A, operator_t& op,
-                                             priority_t& priority, float delta, vertex_t* near0, vertex_t* near1,
-                                             vertex_t* far0, vertex_t* far1, int* queue_stamp, int* far_flag,
-                                             near_far_state_t* state, unsigned long long capacity, int max_levels,
-                                             unsigned long long shrink_limit, unsigned long long grow_limit,
-                                             sync_t sync) {
+template <typename vertex_t, typename edge_t, typename weight_t, typename operator_t, typename priority_t>
+__global__ void __launch_bounds__(256, 2)
+    near_far_kernel(const graph::adjacency_t<vertex_t, edge_t, weight_t> A, operator_t op, priority_t priority,
+                    float delta, vertex_t* near0, vertex_t* near1, vertex_t* far0, vertex_t* far1, int* queue_stamp,
+                    int* far_flag, near_far_state_t* state, unsigned long long capacity, int max_levels) {
+  cooperative_groups::grid_group grid = cooperative_groups::this_grid();
   volatile near_far_state_t* st = state;
   const unsigned lane = b200::lane_id();
   const unsigned long long tid = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -261,8 +245,7 @@ __device__ __forceinline__ void near_far_run(const graph::adjacency_t<vertex_t, 
   vertex_t* near_q[2] = {near0, near1};
   vertex_t* far_q[2] = {far0, far1};
   unsigned long long my_relax = 0;
-  int level = st->level;
-  int reason = near_far_done;
+  int level = 0;
   bool stop = false;
   bool overflowed = false;
 
@@ -289,16 +272,6 @@ __device__ __forceinline__ void near_far_run(const graph::adjacency_t<vertex_t, 
         stop = true;
         break;
       }
-      if (n_in <= shrink_limit) {  // uniform: every thread reads the same value after the barrier
-        stop = true;
-        reason = near_far_shrank;
-        break;
-      }
-      if (grow_limit && n_in > grow_limit) {
-        stop = true;
-        reason = near_far_grew;
-        break;
-      }
       const vertex_t* q_in = near_q[level & 1];
       vertex_t* q_out = near_q[(level + 1) & 1];
       unsigned long long* out_count = &state->near_count[(level + 1) % 3];
@@ -310,7 +283,7 @@ __device__ __forceinline__ void near_far_run(const graph::adjacency_t<vertex_t, 
       if (tid == 0) st->near_count[(level + 2) % 3] = 0;  // consumed a level ago; the next level appends to it
       near_far_expand_level(A, op, priority, q_in, n_in, q_out, out_count, far_out, far_count, threshold, next_level,
                             queue_stamp, far_flag, capacity, tid, threads, my_relax, overflowed);
-      sync();
+      grid.sync();
       ++level;
     }
     if (stop) break;
@@ -319,10 +292,6 @@ __device__ __forceinline__ void near_far_run(const graph::adjacency_t<vertex_t, 
     const int fsel = st->far_selector;
     const unsigned long long n_far = st->far_count[fsel];
     if (n_far == 0) break;
-    if (grow_limit && n_far > 64 * grow_limit) {
-      reason = near_far_grew;
-      break;
-    }
     const vertex_t* far_in = far_q[fsel];
     vertex_t* far_keep = far_q[fsel ^ 1];
     {
@@ -337,7 +306,7 @@ __device__ __forceinline__ void near_far_run(const graph::adjacency_t<vertex_t, 
       }
       if (lane == 0 && lowest != near_far_inf_bits) atomicMin(&state->far_min_bits, lowest);
     }
-    sync();
+    grid.sync();
     const float old_threshold = st->threshold;
     const float far_min = __uint_as_float(st->far_min_bits);
     float new_threshold = (floorf(far_min / delta) + 1.0f) * delta;
@@ -369,7 +338,7 @@ __device__ __forceinline__ void near_far_run(const graph::adjacency_t<vertex_t, 
         append(keep, u, far_keep, keep_count);
       }
     }
-    sync();
+    grid.sync();
     if (tid == 0) {
       st->threshold = new_threshold;
       st->far_count[fsel] = 0;
@@ -377,66 +346,16 @@ __device__ __forceinline__ void near_far_run(const graph::adjacency_t<vertex_t, 
       st->far_min_bits = near_far_inf_bits;
       st->splits = st->splits + 1;
     }
-    sync();
+    grid.sync();
   }
 
   my_relax = b200::warp_sum(my_relax);
   if (lane == 0 && my_relax) atomicAdd(&state->relaxations, my_relax);
   if (overflowed) state->overflow = 1;
-  if (tid == 0) {
-    st->levels = level;
-    st->level = level;
-    st->exit_reason = reason;
-  }
-}
-
-/// Grid-wide form: cooperative launch, one CTA of 256 threads per SM (knob), barrier = cooperative-groups grid sync.
-template <typename vertex_t, typename edge_t, typename weight_t, typename operator_t, typename priority_t>
-__global__ void __launch_bounds__(256, 2)
-    near_far_kernel(const graph::adjacency_t<vertex_t, edge_t, weight_t> A, operator_t op, priority_t priority,
-                    float delta, vertex_t* near0, vertex_t* near1, vertex_t* far0, vertex_t* far1, int* queue_stamp,
-                    int* far_flag, near_far_state_t* state, unsigned long long capacity, int max_levels,
-                    unsigned long long shrink_limit) {
-  cooperative_groups::grid_group grid = cooperative_groups::this_grid();
-  near_far_run(A, op, priority, delta, near0, near1, far0, far1, queue_stamp, far_flag, state, capacity, max_levels,
-               shrink_limit, 0ull, [&]() { grid.sync(); });
-}
-
-/**
- * @brief The same traversal run by ONE thread-block cluster (8 or 16 CTAs x 1024 threads on neighbouring SMs), for
- * levels of at most a few ten thousand vertices (the 4900 x 4900 grid never has more than ~10 K in a level, over
- * ~12.6 K levels): 16 K threads are still a thread per queued vertex there, and the level barrier is the hardware
- * barrier.cluster instead of a 148-CTA cooperative grid sync.
- */
-template <typename vertex_t, typename edge_t, typename weight_t, typename operator_t, typename priority_t>
-__global__ void __launch_bounds__(1024, 1)
-    near_far_cluster_kernel(const graph::adjacency_t<vertex_t, edge_t, weight_t> A, operator_t op, priority_t priority,
-                            float delta, vertex_t* near0, vertex_t* near1, vertex_t* far0, vertex_t* far1,
-                            int* queue_stamp, int* far_flag, near_far_state_t* state, unsigned long long capacity,
-                            int max_levels, unsigned long long grow_limit) {
-  cooperative_groups::cluster_group cluster = cooperative_groups::this_cluster();
-  near_far_run(A, op, priority, delta, near0, near1, far0, far1, queue_stamp, far_flag, state, capacity, max_levels,
-               0ull, grow_limit, [&]() { cluster.sync(); });
+  if (tid == 0) st->levels = level;
 }
 
 }  // namespace kernels
-
-/// Development knob: CTAs per SM of the persistent kernel (fewer CTAs = cheaper grid barrier).
-inline int& near_far_ctas_per_sm() {
-  static int ctas = 1;  // measured on the 4900^2 grid: 1 CTA/SM 178 ms, 2: 192 ms, 4: 232 ms (barrier cost)
-  return ctas;
-}
-
-/// Knob (ess_tune "near_far_cluster"): run levels of at most 64 K vertices in ONE thread-block cluster (hardware
-/// barrier.cluster) and hand larger ones to the grid-wide kernel. Default OFF: on BASELINE config 3 (4900^2 grid,
-/// ~10 K vertices per level) the cluster kernel measured 11.9 us per level against 9.25 us for the grid-wide kernel
-/// (profiles/r02i_probe_grid.log): a level issues ~80 K global atomics (label min + stamp exchange), and 16 SMs'
-/// load/store units take longer to issue them than 148 SMs take to cross a cooperative grid barrier. Both paths
-/// stay tested (test_sssp_near_far_cluster_and_grid_kernels_agree).
-inline int& near_far_cluster_enabled() {
-  static int enabled = 0;
-  return enabled;
-}
 
 /// Statistics of one execute_near_far call.
 struct near_far_result_t {
@@ -483,80 +402,26 @@ near_far_result_t execute_near_far(graph_t& G, enactor_type* E, operator_t op, p
   h.far_min_bits = kernels::near_far_inf_bits;
   cudaMemcpyAsync(state.data(), &h, sizeof(h), cudaMemcpyHostToDevice, stream);
 
-  auto grid_kernel = kernels::near_far_kernel<vertex_t, edge_t, weight_t, operator_t, priority_t>;
-  auto cluster_kernel = kernels::near_far_cluster_kernel<vertex_t, edge_t, weight_t, operator_t, priority_t>;
+  auto kernel = kernels::near_far_kernel<vertex_t, edge_t, weight_t, operator_t, priority_t>;
   int per_sm = 0;
-  error::throw_if_exception(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, grid_kernel, 256, 0), "occupancy");
+  error::throw_if_exception(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, 256, 0), "occupancy");
   error::throw_if_exception(per_sm < 1, "execute_near_far: kernel does not fit on an SM");
-  const int want = near_far_ctas_per_sm();
-  const unsigned grid = unsigned(ctx->sm_count()) * unsigned(per_sm < want ? per_sm : want);
-  // one cluster of 16 CTAs (non-portable size) when the device schedules it, else 8; 0 = no cluster path
-  int cluster_ctas = 0;
-  if (near_far_cluster_enabled()) {
-    for (int size : {16, 8}) {
-      cudaLaunchConfig_t probe{};
-      probe.gridDim = dim3(unsigned(size));
-      probe.blockDim = dim3(1024);
-      cudaLaunchAttribute attr{};
-      attr.id = cudaLaunchAttributeClusterDimension;
-      attr.val.clusterDim.x = unsigned(size);
-      attr.val.clusterDim.y = attr.val.clusterDim.z = 1;
-      probe.attrs = &attr;
-      probe.numAttrs = 1;
-      if (size > 8 && cudaFuncSetAttribute(cluster_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) !=
-                          cudaSuccess) {
-        cudaGetLastError();
-        continue;
-      }
-      int clusters = 0;
-      if (cudaOccupancyMaxActiveClusters(&clusters, cluster_kernel, &probe) == cudaSuccess && clusters >= 1) {
-        cluster_ctas = size;
-        break;
-      }
-      cudaGetLastError();
-    }
-  }
-  const unsigned long long grow_limit = 4ull * 1024ull * unsigned(cluster_ctas);   // cluster -> grid above this
-  const unsigned long long shrink_limit = cluster_ctas ? grow_limit / 4 : 0ull;    // grid -> cluster at or below this
+  // one CTA per SM: the fewer CTAs, the cheaper the grid barrier (4900^2 grid: 178 ms at 1 CTA/SM, 192 ms at 2,
+  // 232 ms at 4)
+  const unsigned grid = unsigned(ctx->sm_count());
   auto adjacency = A;
   vertex_t *near0 = in->data(), *near1 = out->data(), *f0 = far0.data(), *f1 = far1.data();
   int *stamp_ptr = stamp.data(), *flag_ptr = far_flag.data();
   near_far_state_t* state_ptr = state.data();
   unsigned long long capacity = n;
-  bool use_cluster = cluster_ctas > 0 && nf <= grow_limit;
+  void* args[] = {&adjacency, &op, &priority, &delta, &near0, &near1, &f0, &f1, &stamp_ptr, &flag_ptr, &state_ptr,
+                  &capacity, &max_levels};
   ctx->profiler().begin(gcuda::profiler_t::push_expand, stream);
-  int launches = 0;
-  for (;;) {
-    if (use_cluster) {
-      cudaLaunchConfig_t cfg{};
-      cfg.gridDim = dim3(unsigned(cluster_ctas));
-      cfg.blockDim = dim3(1024);
-      cfg.stream = stream;
-      cudaLaunchAttribute attr{};
-      attr.id = cudaLaunchAttributeClusterDimension;
-      attr.val.clusterDim.x = unsigned(cluster_ctas);
-      attr.val.clusterDim.y = attr.val.clusterDim.z = 1;
-      cfg.attrs = &attr;
-      cfg.numAttrs = 1;
-      error::throw_if_exception(cudaLaunchKernelEx(&cfg, cluster_kernel, adjacency, op, priority, delta, near0, near1,
-                                                   f0, f1, stamp_ptr, flag_ptr, state_ptr, capacity, max_levels,
-                                                   grow_limit),
-                                "execute_near_far cluster launch");
-    } else {
-      unsigned long long limit = shrink_limit;
-      void* args[] = {&adjacency, &op,   &priority,  &delta,    &near0,     &near1,    &f0,
-                      &f1,        &stamp_ptr, &flag_ptr, &state_ptr, &capacity, &max_levels, &limit};
-      error::throw_if_exception(
-          cudaLaunchCooperativeKernel((void*)grid_kernel, dim3(grid), dim3(256), args, 0, stream),
-          "execute_near_far launch");
-    }
-    ++launches;
-    cudaMemcpyAsync(&h, state.data(), sizeof(h), cudaMemcpyDeviceToHost, stream);
-    ctx->synchronize();
-    if (h.overflow != 0 || h.exit_reason == kernels::near_far_done) break;
-    use_cluster = h.exit_reason == kernels::near_far_shrank;
-  }
-  ctx->profiler().end(stream, launches);
+  error::throw_if_exception(cudaLaunchCooperativeKernel((void*)kernel, dim3(grid), dim3(256), args, 0, stream),
+                            "execute_near_far launch");
+  cudaMemcpyAsync(&h, state.data(), sizeof(h), cudaMemcpyDeviceToHost, stream);
+  ctx->synchronize();
+  ctx->profiler().end(stream);
   error::throw_if_exception(h.overflow != 0, "execute_near_far: queue overflow");
   in->set_number_of_elements(0);
   out->set_number_of_elements(0);

@@ -10,9 +10,8 @@
  * visited set and the walk stops. Frontier, next frontier and visited set are 1-bit-per-vertex maps: at
  * scale-26 each is 8 MiB and stays in the 126 MB L2, so the per-edge membership probe never reaches HBM.
  *
- * Mapping: one warp per 32-vertex word. A fully visited word costs one 4-byte read; otherwise lanes read
- * their row bounds coalesced, walk their lists, and a ballot assembles the next-frontier word, so dense
- * outputs are written without atomics.
+ * Mapping: one warp per 1024-vertex chunk (pull_chunk_kernel); next-frontier and visited words are assembled in
+ * shared memory and leave as coalesced stores.
  */
 #pragma once
 
@@ -72,149 +71,27 @@ __global__ void __launch_bounds__(256)
   if (b200::lane_id() == 0 && mine) atomicAdd(counters + scratch_t::aux2, mine);
 }
 
-/**
- * @brief One bottom-up level. counters[out_count] += |next frontier|, counters[aux2] += Σdeg(next frontier),
- * counters[aux0] += unvisited vertices walked, counters[aux1] += in-edges read (work accounting).
- * `A` is the CSC adjacency (for a symmetric graph it aliases the CSR arrays).
- *
- * One warp per 32-vertex word, one lane per vertex. What ncu showed for the straightforward version
- * (profiles/r01_pull_step_full_raw.csv, r01_pull_sass_hotspots.txt): DRAM at 19 % of peak, 45 % issue
- * utilisation, and 70 % of the stall samples on two instructions — the consumer of the frontier-bit probe
- * (an L2 round trip) and the consumer of the operator's atomicMin. Neither bandwidth nor trip count is
- * the limit (a 4-words-per-warp version, a warp-cooperative version and a compacted-candidate-list version
- * were all slower or equal). So this version shortens the per-trip dependency chain:
- *   - software pipeline, depth 2: the visited word, row bounds and head hint of the warp's words t+1, t+2 and
- *     the frontier-bit probe of word t+1 are in flight while word t is processed;
- *   - head hint (graph::build::pull_hints): the highest-degree in-neighbour is read coalesced next to the row
- *     bounds and resolves ~85 % of the vertices of a Kronecker BFS without touching the adjacency list;
- *   - the operator's pull form (directional_operator_t) replaces the atomic round trip by a store;
- *   - 32-bit index arithmetic and counters (vertex ids are int32).
- * Semantics: the hinted in-neighbour is offered first, then the in-edges in order, until the operator
- * returns true.
- */
-template <typename vertex_t, typename edge_t, typename weight_t, typename operator_t>
-__global__ void __launch_bounds__(256, 6)
-    pull_step_kernel(const graph::adjacency_t<vertex_t, edge_t, weight_t> A, operator_t op,
-                     const unsigned* __restrict__ frontier_bits, unsigned* __restrict__ next_bits,
-                     unsigned* __restrict__ visited, counter_t* counters) {
-  // Multi-GPU use: A may hold only the rows of a contiguous range of global vertices; `visited` and `next_bits`
-  // then point at the words of that range, frontier_bits and the neighbour ids stay global, and the operator
-  // receives the LOCAL row index as destination.
-  const unsigned lane = b200::lane_id();
-  const unsigned n = unsigned(A.n);
-  const unsigned n_words = (n + 31u) >> 5;
-  const unsigned warps = (gridDim.x * blockDim.x) >> 5;
-  const bool hinted = A.head != nullptr;
-  unsigned found_vertices = 0, scanned = 0, inspected = 0;
-  counter_t found_edges = 0;
-
-  struct stage_t {
-    unsigned seen;
-    edge_t beg, end;
-    vertex_t head;
-  };
-  auto load_seen = [&](unsigned w) -> unsigned { return w < n_words ? visited[w] : 0xffffffffu; };
-  // row bounds + hint of this lane's vertex of word w — only for lanes whose visited bit is clear, so fully
-  // or mostly visited words (isolated vertices, late levels) cost no row/hint traffic
-  auto load_stage = [&](unsigned w, unsigned seen) {
-    stage_t s{seen, 0, 0, vertex_t(-1)};
-    if (!((seen >> lane) & 1u)) {  // padding lanes of the last word are marked visited by init_visited_kernel
-      const unsigned v = (w << 5) + lane;
-      s.beg = A.offsets[v];
-      s.end = A.offsets[v + 1];
-      if (hinted) s.head = hint_vertex(__ldg(A.head + v));
-    }
-    return s;
-  };
-  auto probe_of = [&](const stage_t& s) -> unsigned {  // frontier word holding the head of this lane's vertex
-    return s.head >= 0 ? __ldg(frontier_bits + (unsigned(s.head) >> 5)) : 0u;
-  };
-
-  // software pipeline over the warp's words w, w+warps, ...:  visited word 3 trips ahead, row bounds + hint
-  // 2 trips ahead, frontier probe 1 trip ahead
-  unsigned w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  stage_t cur = load_stage(w, load_seen(w));
-  stage_t nxt = load_stage(w + warps, load_seen(w + warps));
-  unsigned seen_far = load_seen(w + 2 * warps);
-  unsigned probe = probe_of(cur);
-  while (w < n_words) {
-    const unsigned seen_farther = load_seen(w + 3 * warps);
-    const stage_t far = load_stage(w + 2 * warps, seen_far);
-    const unsigned probe_next = probe_of(nxt);
-    bool found = false;
-    if (!((cur.seen >> lane) & 1u)) {
-      ++scanned;
-      const vertex_t v = vertex_t((w << 5) + lane);
-      bool head_tried = false;
-      if (cur.head >= 0 && ((probe >> (unsigned(cur.head) & 31u)) & 1u)) {
-        const edge_t edge = __ldg(A.head_edge + v);
-        const weight_t weight = A.values ? __ldg(A.values + edge) : weight_t(1);
-        found = call_pull(op, cur.head, v, edge, weight);
-        head_tried = true;
-      }
-      for (edge_t e = cur.beg; e < cur.end && !found; ++e) {
-        ++inspected;
-        const vertex_t u = __ldg(A.indices + e);
-        if (head_tried && u == cur.head) continue;  // already offered to the operator
-        if ((__ldg(frontier_bits + (unsigned(u) >> 5)) >> (unsigned(u) & 31u)) & 1u) {
-          const weight_t weight = A.values ? __ldg(A.values + e) : weight_t(1);
-          found = call_pull(op, u, v, e, weight);
-        }
-      }
-    }
-    const unsigned fresh = __ballot_sync(b200::full_mask, found);
-    if (lane == 0) {
-      next_bits[w] = fresh;
-      if (fresh) visited[w] = cur.seen | fresh;
-      found_vertices += __popc(fresh);
-    }
-    if (found) found_edges += counter_t(cur.end - cur.beg);
-    w += warps;
-    cur = nxt;
-    nxt = far;
-    seen_far = seen_farther;
-    probe = probe_next;
-  }
-  found_edges = b200::warp_sum(found_edges);
-  scanned = b200::warp_sum(scanned);
-  inspected = b200::warp_sum(inspected);
-  if (lane == 0) {
-    if (found_vertices) atomicAdd(counters + scratch_t::out_count, counter_t(found_vertices));
-    if (found_edges) atomicAdd(counters + scratch_t::aux2, found_edges);
-    if (scanned) atomicAdd(counters + scratch_t::aux0, counter_t(scanned));
-    if (inspected) atomicAdd(counters + scratch_t::aux1, counter_t(inspected));
-  }
-}
-
 /// A chunk is 32 words = 1024 vertices: what one warp takes per trip of pull_chunk_kernel.
 constexpr int pull_chunk_words = 32;
 constexpr int pull_queue_cap = 32 + 4 * 32;  ///< walk queue of a warp: < 32 left over + one 4-batch group of misses
 constexpr int pull_long_list = 64;           ///< adjacency lists longer than this are walked by the whole warp
 
 /**
- * @brief One bottom-up level, second design (same contract as pull_step_kernel minus the Σdeg of the next
- * frontier: counters[out_count] += |next frontier|, counters[aux0] += unvisited vertices probed,
- * counters[aux1] += in-edges read, counters[aux2] += vertices whose adjacency was walked).
+ * @brief One bottom-up level. Counters: counters[out_count] += |next frontier|, counters[aux0] += unvisited vertices
+ * probed, counters[aux1] += in-edges read, counters[aux2] += vertices whose adjacency was walked. The row bounds of
+ * adopted vertices are not read, so Σdeg of the next frontier is not produced.
+ * Semantics: for each unvisited vertex, the hinted in-neighbour is offered to the operator first, then the in-edges
+ * in list order, until the operator returns true.
+ * `A` is the CSC adjacency (for a symmetric graph it aliases the CSR arrays). It may cover a contiguous row range
+ * that starts at a multiple of 32 (a partitioned graph's owned rows): `visited` and `next_bits` then point at that
+ * range's words, `frontier_bits` and the neighbour ids stay global, and the operator receives the LOCAL row index as
+ * destination.
  *
- * Why a second design. ncu on pull_step_kernel (profiles/r01c_pull_step_summary.txt): 223 warp instructions per
- * 32-vertex word at 12-17 active lanes per instruction, DRAM traffic 3.1x the algorithmic bytes. A CPU model of the
- * same levels (Kronecker scale 20-22) shows why: the head hint resolves 76-99 % of the probed vertices, and 56-99 %
- * of the vertices it does not resolve have a single in-edge — the hint WAS their whole adjacency — so the warp
- * spent most of its instructions in a walk loop that 2-5 of its 32 lanes were executing, re-reading a neighbour it
- * already knew, and it paid the row bounds (2 x sizeof(edge_t), one random sector) for every probed vertex although
- * only real walks need them.
- *   compaction: a warp takes a chunk of 32 words; lane L loads visited word L (one coalesced 128-byte access) and
- *     the chunk's unvisited vertices are compacted into shared memory (shuffle scan of the popcounts), so every
- *     later instruction runs with 32 busy lanes however sparse the level is.
- *   hint phase: the compacted vertices are taken 4 x 32 at a time: 4 head loads -> 4 frontier-word probes ->
- *     operator (owner-exclusive form); found bits are ORed into the chunk's 32 result words in shared memory. No row
- *     bounds are read. Single-in-edge vertices whose hint missed are finished. The others join the walk queue.
- *   walk: whenever 32 vertices are queued they are walked one per lane, all lanes busy: row bounds on demand, the
- *     list read until the operator returns true. Lists longer than pull_long_list are left to a warp-cooperative
- *     pass (coalesced 32-edge strides, ballot, candidates offered in list order).
- *   write-back: next/visited words of the chunk leave shared memory as one coalesced store each.
- * Semantics: hinted in-neighbour first, then the in-edges in list order, until the operator returns true — as
- * pull_step_kernel. Single-GPU form (A holds every row; visited/next are full-length).
+ * Why it looks as it does: a warp-per-word walk ran most of its instructions with 2-5 busy lanes and read row bounds
+ * for every probed vertex, though the head hint alone settles most of them (DESIGN.md §3.2). So the chunk's unvisited
+ * vertices are compacted into shared memory (all 32 lanes busy however sparse the level), the hints are probed
+ * 4 x 32 at a time without row bounds, and only hint misses with more than one in-edge join a walk queue, drained
+ * 32 at a time; lists longer than pull_long_list are walked by the whole warp in coalesced 32-edge strides.
  */
 template <typename vertex_t, typename edge_t, typename weight_t, typename operator_t>
 __global__ void __launch_bounds__(256, 5)
@@ -391,12 +268,6 @@ __global__ void __launch_bounds__(256, 5)
     if (inspected) atomicAdd(counters + scratch_t::aux1, counter_t(inspected));
     if (walked) atomicAdd(counters + scratch_t::aux2, counter_t(walked));  // vertices whose adjacency was walked
   }
-}
-
-/// Development knob (ess_tune "pull_engine"): 1 = pull_chunk_kernel (default), 0 = pull_step_kernel.
-inline int& pull_engine() {
-  static int engine = 1;
-  return engine;
 }
 
 /// Development knob: use the per-vertex head hints when the graph carries them (default on).

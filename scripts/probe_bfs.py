@@ -18,7 +18,7 @@ ap.add_argument("--pull-variants", default="")
 ap.add_argument("--hints", default="1")
 ap.add_argument("--alphas", default="0")
 ap.add_argument("--betas", default="0")
-ap.add_argument("--engines", default="11", help="comma list of <advance_engine><pull_engine> digits, e.g. 00,11")
+ap.add_argument("--engines", default="1", help="comma list of advance_engine values: 1 quad engine, 0 scalar kernels")
 args = ap.parse_args()
 
 t = time.time()
@@ -38,8 +38,7 @@ runs = [(v, pv, int(h), float(a), float(b), eng) for eng in args.engines.split("
 for variant, pv, hints, alpha, beta, eng in runs:
     lb, direction = variant.split(":")
     ess.tune("pull_hints", hints)
-    ess.tune("advance_engine", int(eng[0]))
-    ess.tune("pull_engine", int(eng[1]))
+    ess.tune("advance_engine", int(eng))
     variant = f"{variant}/eng{eng}/h{hints}/a{alpha:g}/b{beta:g}"
     for s in srcs:
         ctx.profile(True)

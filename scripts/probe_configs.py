@@ -38,11 +38,8 @@ if not args.skip_sssp:
         print(f"sssp {lb:14s} enact={info['enact_ms']:10.2f} ms iters={info['iterations']} "
               f"GTEPS={csr.m/info['enact_ms']/1e6:.4f}{ok}  "
               + " ".join(f"{k}={v[0]:.1f}ms/{v[1]}" for k, v in prof.items() if v[1]), flush=True)
-    import itertools
-    for ctas, delta in itertools.product((2, 1, 4), (0.0, 512.0, 2048.0, 8192.0)):
-        ess.tune("near_far_ctas", ctas)
+    for delta in (0.0, 512.0, 2048.0, 8192.0):
         dist, info = ess.sssp_near_far(ctx, g, 0, delta=delta)
-        print(f"ctas/SM={ctas} ", end="")
         ok = "" if want is None else f" bit-exact={np.array_equal(dist.cpu().numpy(), want)}"
         print(f"sssp near_far delta={delta:6.1f} enact={info['enact_ms']:10.2f} ms levels={info['levels']} "
               f"splits={info['splits']} relaxations={info['relaxations']} ({info['relaxations']/csr.m:.2f} x m) "

@@ -1,6 +1,6 @@
 """CPU suite: the multi-GPU BFS host logic (1-D partition, bitmap exchange, direction switch, termination) on
 world_size 2 and 4 with the gloo backend. The per-rank level kernels are replaced by a numpy stand-in with
-the same contract as ess_bfs_partition_step / ess_bfs_absorb (this double lives in tests/, not the product)."""
+the same contract as ess_bfs_partition_step / ess_bfs_partition_pull / ess_bfs_absorb (this double lives in tests/, not the product)."""
 import os
 import socket
 
@@ -44,9 +44,7 @@ class NumpyBackend:
         visited[lo:lo + self.n_local] |= found
         self._store(visited_bits, visited, 0)
         self._store(next_slice, found, 0)
-        deg = np.diff(self.off)
-        counts.view(torch.int64)[0] += int(found.sum())
-        counts.view(torch.int64)[1] += int(deg[found].sum())
+        counts.view(torch.int64)[0] += int(found.sum())  # counts[1] untouched, as ess_bfs_partition_pull
 
     def merge(self, gathered, world, slice_words, frontier_bits, visited_bits, counts_out):
         rows = gathered.view(world, slice_words + 4)

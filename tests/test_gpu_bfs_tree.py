@@ -4,8 +4,8 @@ Contract, for a run from `source` with `depth` exactly as ess.bfs returns it: pr
 exactly where depth[v] == INT32_MAX; every other pred[v] is in [0, n), is the tail of an edge pred[v] -> v of the CSR
 and has depth[pred[v]] == depth[v] - 1. Which valid parent is chosen is not deterministic, so the tests check these
 rules, never a particular tree, and they compare the depths bit for bit with ess.bfs, the golden vectors or the
-oracle. Every balancer runs forward and direction-optimised, including the fallback kernels (pull_engine 0,
-pull_hints 0, advance_engine 0, a misaligned graph), on caller buffers that hold garbage, start 4 bytes past a
+oracle. Every balancer runs forward and direction-optimised, including the fallback kernels (pull_hints 0,
+advance_engine 0, a misaligned graph), on caller buffers that hold garbage, start 4 bytes past a
 16-byte boundary or are reused across sources."""
 import importlib.util
 import os
@@ -23,7 +23,7 @@ pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LBS = list(ess.IMPLEMENTED_LOAD_BALANCERS)
 INT32_MAX = np.iinfo(np.int32).max
-KNOB_DEFAULTS = {"advance_engine": 1, "pull_engine": 1, "pull_hints": 1, "sssp_fused_unique": 1}
+KNOB_DEFAULTS = {"advance_engine": 1, "pull_hints": 1, "sssp_fused_unique": 1}
 
 
 def _load_cost_script():
@@ -169,13 +169,12 @@ def test_rmat16_trees(ctx, s16, lb):
                 assert info["pull_steps"] >= 1 and info["pull_found"] > 0, (s, lb, info)
 
 
-FALLBACKS = [("pull_engine", 0), ("pull_hints", 0), ("advance_engine", 0)]
+FALLBACKS = [("pull_hints", 0), ("advance_engine", 0)]
 
 
 @pytest.mark.parametrize("name,value", FALLBACKS)
 def test_trees_on_the_fallback_kernels(ctx, s16, name, value):
-    """The old bottom-up kernel (its head-hint path included), bottom-up without hints and the scalar advance
-    kernels: RMAT scale 16 and arbitrary directed multigraphs."""
+    """Bottom-up without hints and the scalar advance kernels: RMAT scale 16 and arbitrary directed multigraphs."""
     csr, g, (off, col, _) = s16
     rng = np.random.default_rng(31)
     with knob(name, value):

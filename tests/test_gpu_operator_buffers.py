@@ -4,7 +4,7 @@ The algorithm tests elsewhere run every operator on buffers the library sized it
 operators what a caller may pass instead: output buffers of every capacity around the frontier's worst case
 (Σdeg), graph arrays freed and rebuilt at the same address, and tensor views that start 4 bytes past a 16-byte
 boundary. They also run the fallback kernels that only a knob or a misaligned graph selects: the scalar advance
-kernels (advance_engine 0), the old bottom-up kernel (pull_engine 0) and bottom-up without hints (pull_hints 0).
+kernels (advance_engine 0) and bottom-up without hints (pull_hints 0).
 Every expected value comes from NumPy or the CPU oracle."""
 import numpy as np
 import pytest
@@ -19,7 +19,7 @@ pytestmark = pytest.mark.gpu
 LBS = list(ess.IMPLEMENTED_LOAD_BALANCERS)
 BIG_DEGREE = 4096  # kernels::big_degree: lists this long are expanded grid-wide (bucketing's third bin)
 WARP_DEGREE = 32   # kernels::warp_degree: bucketing gives lists this long a warp
-KNOB_DEFAULTS = {"advance_engine": 1, "pull_engine": 1, "pull_hints": 1, "sssp_fused_unique": 1}
+KNOB_DEFAULTS = {"advance_engine": 1, "pull_hints": 1, "sssp_fused_unique": 1}
 
 
 @pytest.fixture(scope="module")
@@ -381,7 +381,7 @@ def _arbitrary_multigraph(rng):
     return _csr(off, col, val, "arbitrary", False)
 
 
-FALLBACKS = [("pull_engine", 0), ("pull_hints", 0), ("advance_engine", 0)]
+FALLBACKS = [("pull_hints", 0), ("advance_engine", 0)]
 
 
 @pytest.fixture(scope="module")
@@ -392,8 +392,7 @@ def s16():
 
 @pytest.mark.parametrize("name,value", FALLBACKS)
 def test_optimized_bfs_fallbacks(ctx, s16, name, value):
-    """Direction-optimised BFS with the old bottom-up kernel, without the bottom-up hints, and with the scalar
-    advance kernels: bit-equal to the oracle on RMAT scale 16 (which must switch to bottom-up) and on arbitrary
+    """Direction-optimised BFS without the bottom-up hints and with the scalar advance kernels: bit-equal to the oracle on RMAT scale 16 (which must switch to bottom-up) and on arbitrary
     directed multigraphs (CSR + transposed CSC)."""
     csr, g, (off, col, _) = s16
     rng = np.random.default_rng(21)

@@ -218,25 +218,19 @@ def test_sssp_near_far_larger_graphs(ctx):
         assert info["relaxations"] >= grid.m * 0 + 1
 
 
-@pytest.mark.parametrize("cluster", [0, 1])
-def test_sssp_near_far_cluster_and_grid_kernels_agree(ctx, cluster):
-    """execute_near_far runs small levels in one thread-block cluster (DSMEM counters, hardware cluster barrier) and
-    hands over to the grid-wide cooperative kernel when a level outgrows the cluster, and back: same distances from
-    either kernel alone (knob 0) and from the mixed run (a Kronecker graph crosses the hand-over limits both ways)."""
-    ess.tune("near_far_cluster", cluster)
-    try:
-        grid = gg.grid_csr(211, 97, device="cuda")
-        off, col, val = grid.host()
-        dist, info = ess.sssp_near_far(ctx, ess.Graph(grid), 5)
-        assert np.array_equal(dist.cpu().numpy(), oracle.sssp(off, col, val, 5))
-        assert info["levels"] > 200
-        csr = gg.rmat_csr(17, weights="hash", device="cuda")  # levels far beyond 64 K vertices: grid-wide kernel
-        off, col, val = csr.host()
-        s = gg.pick_sources(csr, 1)[0]
-        dist, info = ess.sssp_near_far(ctx, ess.Graph(csr), s)
-        assert np.array_equal(dist.cpu().numpy(), oracle.sssp(off, col, val, s))
-    finally:
-        ess.tune("near_far_cluster", 0)
+def test_sssp_near_far_long_runs(ctx):
+    """One launch of the persistent near-far kernel over hundreds of small levels (a long, thin grid) and over the wide
+    levels of a Kronecker graph: distances bit-equal to the oracle."""
+    grid = gg.grid_csr(211, 97, device="cuda")
+    off, col, val = grid.host()
+    dist, info = ess.sssp_near_far(ctx, ess.Graph(grid), 5)
+    assert np.array_equal(dist.cpu().numpy(), oracle.sssp(off, col, val, 5))
+    assert info["levels"] > 200
+    csr = gg.rmat_csr(17, weights="hash", device="cuda")
+    off, col, val = csr.host()
+    s = gg.pick_sources(csr, 1)[0]
+    dist, info = ess.sssp_near_far(ctx, ess.Graph(csr), s)
+    assert np.array_equal(dist.cpu().numpy(), oracle.sssp(off, col, val, s))
 
 
 def test_sssp_thresholds_make_progress_on_extreme_weight_ranges(ctx):
