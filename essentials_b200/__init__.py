@@ -81,6 +81,7 @@ _SIGNATURES = {
     "ess_sssp": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_int, POINTER(RunInfo)]),
     "ess_sssp_near_far": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_float, POINTER(RunInfo)]),
     "ess_sssp_delta": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_float, POINTER(RunInfo)]),
+    "ess_sssp_tree": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_void_p, POINTER(RunInfo)]),
     "ess_pagerank": (c_int, [c_void_p, c_void_p, c_float, c_float, c_int, c_void_p, c_int, c_int, POINTER(RunInfo)]),
     "ess_ppr": (c_int, [c_void_p, c_void_p, c_int32, c_float, c_float, c_void_p, c_int, POINTER(RunInfo)]),
     "ess_kcore": (c_int, [c_void_p, c_void_p, c_void_p, c_int, POINTER(RunInfo)]),
@@ -297,11 +298,13 @@ def bfs(ctx: Context, g: Graph, source: int, lb: str = "block_mapped", direction
     return depth, info.as_dict()
 
 
-def _label_buffer(t, g: Graph, what: str):
+def _label_buffer(t, g: Graph, what: str, dtype=None):
     import torch
-    if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.int32 and t.is_contiguous()
+    dtype = torch.int32 if dtype is None else dtype
+    if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == dtype and t.is_contiguous()
             and t.numel() >= g.n and t.device == g.device):
-        raise EssentialsError(f"{what} must be a contiguous int32 CUDA tensor of at least {g.n} elements on {g.device}")
+        name = str(dtype).replace("torch.", "")
+        raise EssentialsError(f"{what} must be a contiguous {name} CUDA tensor of at least {g.n} elements on {g.device}")
     return t
 
 
@@ -357,6 +360,30 @@ def sssp_delta(ctx: Context, g: Graph, source: int, delta: float = 0.0, out=None
     d.update(rounds=int(info.reserved[0]), threshold_advances=int(info.reserved[1]),
              expanded_vertices=int(info.reserved[2]), passes=int(info.reserved[3]))
     return dist, d
+
+
+def sssp_tree(ctx: Context, g: Graph, source: int, dist, pred_out=None):
+    """gunrock::sssp::build_tree: the shortest-path tree of `dist`, the distances :func:`sssp`, :func:`sssp_near_far`
+    or :func:`sssp_delta` returned for `source` on `g`. Returns (pred[int32], info).
+
+    pred[source] == source; pred[v] == -1 exactly where dist[v] == FLT_MAX; a vertex with a strict tight in-edge
+    (dist[u] < dist[v] == fl(dist[u] + w)) takes the smallest such u; the others take the smallest u of a zero-weight
+    tight edge one flat hop closer to those parents (include/essentials_b200.h states the rule). The tree is a pure
+    function of the graph, `dist` and `source`. `dist` must be a contiguous float32 CUDA tensor of at least g.n
+    elements on the graph's device and is only read; `pred_out`, when given, the same as int32, not overlapping
+    `dist`. Distances that are not the SSSP result for `source` raise EssentialsError naming the violation.
+    info adds flat_rounds (rounds over zero-weight edges) and flat_vertices (vertices parented over one)."""
+    import torch
+    dist = _label_buffer(dist, g, "dist", torch.float32)
+    pred = _out(g.n, torch.int32, g) if pred_out is None else _label_buffer(pred_out, g, "pred_out")
+    span = 4 * g.n
+    if dist.data_ptr() < pred.data_ptr() + span and pred.data_ptr() < dist.data_ptr() + span:
+        raise EssentialsError("sssp_tree: pred_out must not overlap dist")
+    info = RunInfo()
+    _check(lib().ess_sssp_tree(ctx.handle, g.handle, int(source), _p(dist), _p(pred), byref(info)), "ess_sssp_tree")
+    d = info.as_dict()
+    d.update(flat_rounds=int(info.iterations), flat_vertices=int(info.reserved[0]))
+    return pred, d
 
 
 def pagerank(ctx: Context, g: Graph, alpha: float = 0.85, tol: float = 1e-6, max_iterations: int = 1000,

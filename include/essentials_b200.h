@@ -149,6 +149,25 @@ ESS_API int ess_sssp_near_far(ess_context_t ctx, ess_graph_t g, int32_t source, 
 ESS_API int ess_sssp_delta(ess_context_t ctx, ess_graph_t g, int32_t source, float* d_dist, float delta,
                            ess_run_info* info);
 
+/* gunrock::sssp::build_tree: the shortest-path tree of distances an SSSP run returned. d_dist: n x float, read only,
+ * the result of ess_sssp (any lb), ess_sssp_near_far or ess_sssp_delta from `source` on this graph. d_pred: n x int32,
+ * 4-byte aligned, required, must not overlap d_dist; every entry is written. With fl(a + w) the float add SSSP uses
+ * and w the CSR weight (1 without values), an edge u -> v is tight when d[u] < FLT_MAX and d[v] == fl(d[u] + w),
+ * strict when also d[u] < d[v], flat when d[u] == d[v] and u != v. On return:
+ *   d_pred[source] == source;
+ *   d_pred[v] == -1 if and only if d_dist[v] == FLT_MAX (v unreached);
+ *   a reached v with a strict tight in-edge: the smallest tail of its strict tight in-edges;
+ *   any other reached v: with the vertices above as anchors and L(v) the flat hops from the nearest anchor, the
+ *     smallest u with a flat edge u -> v and L(u) == L(v) - 1.
+ * The tree is a pure function of the graph, d_dist and source (no cycles; byte-identical for the three SSSP entry
+ * points, which return bit-identical distances). Only CSR out-edges are read: no CSC view is needed.
+ * The call fails, naming the violation and its count, when d_dist is not the SSSP fixed point for `source`: an entry
+ * that is NaN, negative or +inf, d_dist[source] != 0, an edge with fl(d[u] + w) < d[v] and u reached, or a reached
+ * vertex without a tight path from the source. d_pred is then unspecified. info->enact_ms = the pass (CUDA events),
+ * iterations = flat rounds, reserved[0] = vertices parented over a flat edge. */
+ESS_API int ess_sssp_tree(ess_context_t ctx, ess_graph_t g, int32_t source, const float* d_dist, int32_t* d_pred,
+                          ess_run_info* info);
+
 /* gunrock::pr::run — include/gunrock/algorithms/pr.hxx:183-216 (alpha 0.85, tol 1e-6 in examples/algorithms/pr/pr.cu:55-56).
  * pull != 0 gathers over the CSC view instead of scattering with atomics; it fails when only one of the CSR and
  * CSC views carries edge weights. */
