@@ -82,6 +82,7 @@ _SIGNATURES = {
     "ess_sssp_near_far": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_float, POINTER(RunInfo)]),
     "ess_sssp_delta": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_float, POINTER(RunInfo)]),
     "ess_sssp_tree": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_void_p, POINTER(RunInfo)]),
+    "ess_bc": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_float, c_void_p, POINTER(RunInfo)]),
     "ess_pagerank": (c_int, [c_void_p, c_void_p, c_float, c_float, c_int, c_void_p, c_int, c_int, POINTER(RunInfo)]),
     "ess_ppr": (c_int, [c_void_p, c_void_p, c_int32, c_float, c_float, c_void_p, c_int, POINTER(RunInfo)]),
     "ess_kcore": (c_int, [c_void_p, c_void_p, c_void_p, c_int, POINTER(RunInfo)]),
@@ -384,6 +385,50 @@ def sssp_tree(ctx: Context, g: Graph, source: int, dist, pred_out=None):
     d = info.as_dict()
     d.update(flat_rounds=int(info.iterations), flat_vertices=int(info.reserved[0]))
     return pred, d
+
+
+def bc(ctx: Context, g: Graph, sources=None, scale: float = 1.0, out=None):
+    """gunrock::bc::run: betweenness centrality by Brandes' algorithm (include/essentials_b200.h states the contract).
+    Returns (bc[float32], info).
+
+    bc[v] = scale * sum over the sources s != v of Brandes' dependency delta_s(v), hop counts with edge weights ignored
+    and parallel edges counted as distinct paths. `sources`: None (every vertex: exact BC), an int, a sequence of ints
+    or a CPU integer tensor; a source listed twice counts twice. scale=0.5 gives the undirected convention and the
+    reference's single-source output. The result is byte-identical between runs. Needs a CSC view (a symmetric graph
+    or a caller transpose). `out`, when given, must be a contiguous float32 CUDA tensor of at least g.n elements on the
+    graph's device. info adds sources, levels, reached and edges_gathered (sums over the sources)."""
+    import math
+
+    import numpy as np
+    import torch
+    if sources is None:
+        arr = None
+    else:
+        if isinstance(sources, torch.Tensor):
+            if sources.is_cuda or sources.dtype.is_floating_point or sources.dtype.is_complex \
+                    or sources.dtype == torch.bool:
+                raise EssentialsError("bc: a sources tensor must be a CPU integer tensor")
+            sources = sources.reshape(-1).tolist()
+        elif isinstance(sources, (int, np.integer)):
+            sources = [sources]
+        if not isinstance(sources, (list, tuple, range, np.ndarray)) or not all(
+                isinstance(s, (int, np.integer)) and not isinstance(s, bool) for s in sources):
+            raise EssentialsError("bc: sources must be vertex ids (ints)")
+        arr = np.ascontiguousarray(np.array([int(s) for s in sources], dtype=np.int64))
+        if arr.size == 0:
+            raise EssentialsError("bc: sources is empty (None means every vertex)")
+        if arr.min() < 0 or arr.max() >= g.n:
+            raise EssentialsError(f"bc: source out of range [0, {g.n})")
+        arr = arr.astype(np.int32)
+    if not math.isfinite(float(scale)):
+        raise EssentialsError("bc: scale must be finite")
+    res = _out(g.n, torch.float32, g) if out is None else _label_buffer(out, g, "out", torch.float32)
+    info = RunInfo()
+    ptr = None if arr is None else arr.ctypes.data_as(c_void_p)
+    _check(lib().ess_bc(ctx.handle, g.handle, ptr, 0 if arr is None else int(arr.size), float(scale), _p(res),
+                        byref(info)), "ess_bc")
+    return res, {"enact_ms": float(info.enact_ms), "sources": int(info.iterations), "levels": int(info.reserved[0]),
+                 "reached": int(info.reserved[1]), "edges_gathered": int(info.reserved[2])}
 
 
 def pagerank(ctx: Context, g: Graph, alpha: float = 0.85, tol: float = 1e-6, max_iterations: int = 1000,

@@ -168,6 +168,22 @@ ESS_API int ess_sssp_delta(ess_context_t ctx, ess_graph_t g, int32_t source, flo
 ESS_API int ess_sssp_tree(ess_context_t ctx, ess_graph_t g, int32_t source, const float* d_dist, int32_t* d_pred,
                           ess_run_info* info);
 
+/* gunrock::bc::run: betweenness centrality by Brandes' algorithm over the depths of the direction-optimised BFS
+ * (include/gunrock/algorithms/bc.hxx; needs a CSC view). The graph is taken unweighted: a path is a sequence of CSR
+ * edges, so parallel edges are distinct paths, and self-loops are never on a shortest path. With σ_s(v) the number of
+ * shortest s -> v paths and δ_s(v) = Σ_{v->w, d(w) = d(v)+1} σ_s(v)/σ_s(w) · (1 + δ_s(w)), on return
+ *   d_bc[v] = float(scale · Σ_{s ∈ sources, s != v} δ_s(v))   for every v (n x float, every entry written).
+ * h_sources: HOST array of n_sources vertex ids, summed in list order (a source listed twice counts twice); NULL with
+ * n_sources == 0 means every vertex in id order, which is exact BC. scale 1 gives the raw sum, 0.5 the undirected
+ * convention (each unordered pair once; also the reference's single-source output), 1/((n-1)(n-2)) a normalisation.
+ * σ, δ and the sum are double; the result is a pure function of (graph, sources, scale), byte-identical between runs
+ * and for 32- or 64-bit offsets, host-built and misaligned graphs. Refused before any launch: a null ctx, g or d_bc,
+ * n_sources < 0, n_sources == 0 with non-NULL h_sources, a source out of range, a non-finite scale, a graph without
+ * a CSC view. info->enact_ms = device time of the whole call, iterations = number of sources, reserved[0] Σ levels,
+ * [1] Σ reached vertices, [2] Σ edges gathered by both passes. */
+ESS_API int ess_bc(ess_context_t ctx, ess_graph_t g, const int32_t* h_sources, int64_t n_sources, float scale,
+                   float* d_bc, ess_run_info* info);
+
 /* gunrock::pr::run — include/gunrock/algorithms/pr.hxx:183-216 (alpha 0.85, tol 1e-6 in examples/algorithms/pr/pr.cu:55-56).
  * pull != 0 gathers over the CSC view instead of scattering with atomics; it fails when only one of the CSR and
  * CSC views carries edge weights. */
