@@ -290,9 +290,11 @@ def _out(n, dtype, g):
 
 def bfs(ctx: Context, g: Graph, source: int, lb: str = "block_mapped", direction: str = "forward", out=None,
         alpha: float = 0.0, beta: float = 0.0):
-    """gunrock::bfs::run (reference include/gunrock/algorithms/bfs.hxx:151-176). Returns (depth[int32], info)."""
+    """gunrock::bfs::run (reference include/gunrock/algorithms/bfs.hxx:151-176). Returns (depth[int32], info).
+
+    `out`, when given, must be a contiguous int32 CUDA tensor of at least g.n elements on the graph's device."""
     import torch
-    depth = _out(g.n, torch.int32, g) if out is None else out
+    depth = _out(g.n, torch.int32, g) if out is None else _label_buffer(out, g, "out")
     info = RunInfo()
     _check(lib().ess_bfs(ctx.handle, g.handle, int(source), _p(depth), LOAD_BALANCE[lb], DIRECTION[direction],
                          alpha, beta, byref(info)), "ess_bfs")
@@ -330,18 +332,21 @@ def bfs_tree(ctx: Context, g: Graph, source: int, lb: str = "block_mapped", dire
 
 
 def sssp(ctx: Context, g: Graph, source: int, lb: str = "block_mapped", out=None):
-    """gunrock::sssp::run (reference include/gunrock/algorithms/sssp.hxx:155-185). Returns (dist[float32], info)."""
+    """gunrock::sssp::run (reference include/gunrock/algorithms/sssp.hxx:155-185). Returns (dist[float32], info).
+
+    `out`, when given, must be a contiguous float32 CUDA tensor of at least g.n elements on the graph's device."""
     import torch
-    dist = _out(g.n, torch.float32, g) if out is None else out
+    dist = _out(g.n, torch.float32, g) if out is None else _label_buffer(out, g, "out", torch.float32)
     info = RunInfo()
     _check(lib().ess_sssp(ctx.handle, g.handle, int(source), _p(dist), LOAD_BALANCE[lb], byref(info)), "ess_sssp")
     return dist, info.as_dict()
 
 
 def sssp_near_far(ctx: Context, g: Graph, source: int, delta: float = 0.0, out=None):
-    """SSSP through operators::advance::execute_near_far (near/far ordering in one persistent kernel)."""
+    """SSSP through operators::advance::execute_near_far (near/far ordering in one persistent kernel). `out`, when
+    given, must be a contiguous float32 CUDA tensor of at least g.n elements on the graph's device."""
     import torch
-    dist = _out(g.n, torch.float32, g) if out is None else out
+    dist = _out(g.n, torch.float32, g) if out is None else _label_buffer(out, g, "out", torch.float32)
     info = RunInfo()
     _check(lib().ess_sssp_near_far(ctx.handle, g.handle, int(source), _p(dist), float(delta), byref(info)),
            "ess_sssp_near_far")
@@ -351,9 +356,10 @@ def sssp_near_far(ctx: Context, g: Graph, source: int, delta: float = 0.0, out=N
 
 
 def sssp_delta(ctx: Context, g: Graph, source: int, delta: float = 0.0, out=None):
-    """SSSP through gunrock::sssp::run_delta (dense active set + delta thresholds; for low-diameter graphs)."""
+    """SSSP through gunrock::sssp::run_delta (dense active set + delta thresholds; for low-diameter graphs). `out`,
+    when given, must be a contiguous float32 CUDA tensor of at least g.n elements on the graph's device."""
     import torch
-    dist = _out(g.n, torch.float32, g) if out is None else out
+    dist = _out(g.n, torch.float32, g) if out is None else _label_buffer(out, g, "out", torch.float32)
     info = RunInfo()
     _check(lib().ess_sssp_delta(ctx.handle, g.handle, int(source), _p(dist), float(delta), byref(info)),
            "ess_sssp_delta")
@@ -441,9 +447,10 @@ def pagerank(ctx: Context, g: Graph, alpha: float = 0.85, tol: float = 1e-6, max
     `atomic::add` over the out-edges with balancer `lb`; float additions then arrive in whatever order the hardware
     schedules them, so individual ranks can differ by up to ~1e-4 relative from run to run (1e-6 in L1), exactly as
     the reference's GPU PageRank does. Without an in-edge view the default is the scatter. The gather raises
-    :class:`EssentialsError` when only one of the CSR and the CSC carries edge weights."""
+    :class:`EssentialsError` when only one of the CSR and the CSC carries edge weights. `out`, when given, must be a
+    contiguous float32 CUDA tensor of at least g.n elements on the graph's device."""
     import torch
-    p = _out(g.n, torch.float32, g) if out is None else out
+    p = _out(g.n, torch.float32, g) if out is None else _label_buffer(out, g, "out", torch.float32)
     info = RunInfo()
     if pull is None:
         pull = bool(g.has_csc)
@@ -454,9 +461,10 @@ def pagerank(ctx: Context, g: Graph, alpha: float = 0.85, tol: float = 1e-6, max
 
 def ppr(ctx: Context, g: Graph, seed: int, alpha: float = 0.15, epsilon: float = 1e-6, lb: str = "block_mapped",
         out=None):
-    """gunrock::ppr::run (reference include/gunrock/algorithms/ppr.hxx:150-179)."""
+    """gunrock::ppr::run (reference include/gunrock/algorithms/ppr.hxx:150-179). `out`, when given, must be a
+    contiguous float32 CUDA tensor of at least g.n elements on the graph's device."""
     import torch
-    p = _out(g.n, torch.float32, g) if out is None else out
+    p = _out(g.n, torch.float32, g) if out is None else _label_buffer(out, g, "out", torch.float32)
     info = RunInfo()
     _check(lib().ess_ppr(ctx.handle, g.handle, int(seed), alpha, epsilon, _p(p), LOAD_BALANCE[lb], byref(info)),
            "ess_ppr")
@@ -464,18 +472,20 @@ def ppr(ctx: Context, g: Graph, seed: int, alpha: float = 0.15, epsilon: float =
 
 
 def kcore(ctx: Context, g: Graph, lb: str = "block_mapped", out=None):
-    """gunrock::kcore::run (reference include/gunrock/algorithms/kcore.hxx:202-222)."""
+    """gunrock::kcore::run (reference include/gunrock/algorithms/kcore.hxx:202-222). Returns (core[int32], info).
+    `out`, when given, must be a contiguous int32 CUDA tensor of at least g.n elements on the graph's device."""
     import torch
-    k = _out(g.n, torch.int32, g) if out is None else out
+    k = _out(g.n, torch.int32, g) if out is None else _label_buffer(out, g, "out")
     info = RunInfo()
     _check(lib().ess_kcore(ctx.handle, g.handle, _p(k), LOAD_BALANCE[lb], byref(info)), "ess_kcore")
     return k, info.as_dict()
 
 
 def color(ctx: Context, g: Graph, out=None):
-    """gunrock::color::run (reference include/gunrock/algorithms/color.hxx:155-180)."""
+    """gunrock::color::run (reference include/gunrock/algorithms/color.hxx:155-180). Returns (colour[int32], info).
+    `out`, when given, must be a contiguous int32 CUDA tensor of at least g.n elements on the graph's device."""
     import torch
-    c = _out(g.n, torch.int32, g) if out is None else out
+    c = _out(g.n, torch.int32, g) if out is None else _label_buffer(out, g, "out")
     info = RunInfo()
     _check(lib().ess_color(ctx.handle, g.handle, _p(c), byref(info)), "ess_color")
     return c, info.as_dict()
