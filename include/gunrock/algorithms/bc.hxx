@@ -20,15 +20,16 @@
  * Per source, all on the context's stream:
  *   depths    bfs::run<merge_path, optimized>, unchanged;
  *   order     counting sort of the reached vertices by bucket = depth · 9 + 3 · bin(in-degree) + bin(out-degree),
- *             bin = [0, 8) one thread, [8, 4096) one warp, [4096, ∞) one CTA per row (pr.hxx's pull bins):
+ *             bin = b200::degree_bin: [0, 8) one thread, [8, 4096) one warp, [4096, ∞) one CTA per row:
  *             level_histogram_kernel, level_scan_kernel, level_scatter_kernel, then one read-back of the bucket
  *             offsets, which sizes the launches;
  *   forward   levels 1..D, rows binned by in-degree: σ(v) = Σ_{u->v, d(u) = d(v)-1} σ(u) over the CSC, σ(s) = 1;
  *   backward  levels D..0, rows binned by out-degree: δ(v) = σ(v) · Σ_{v->w, d(w) = d(v)+1} c(w) over the CSR, then
  *             c(v) = (1 + δ(v)) / σ(v) and acc[v] += δ(v) for v != s (at level D the sum is empty: c = 1/σ).
- * Both gathers are level_gather_kernel: it reads the 4-byte depth of a neighbour before its 8-byte value, so an edge
- * into another level costs 4 bytes. After the last source one streaming kernel writes bc. Scratch: depth, level order
- * (int32), σ, c, acc (double) — 32 bytes per vertex from the device pool, once per call — and 9 counters per level.
+ * Both gathers are b200::row_gather with level_sum_t, which reads the 4-byte depth of a neighbour before its 8-byte
+ * value, so an edge into another level costs 4 bytes. After the last source one streaming kernel writes bc. Scratch:
+ * depth, level order (int32), σ, c, acc (double) — 32 bytes per vertex from the device pool, once per call — and 9
+ * counters per level.
  *
  * Needs a CSC view (a symmetric graph or a caller transpose), like direction-optimised BFS. σ is a double: it
  * overflows past ~1.8e308 shortest paths (e.g. grids with more than about 1000 hops between corners), and the
@@ -44,19 +45,14 @@
 #include <vector>
 
 #include <gunrock/algorithms/bfs.hxx>
+#include <gunrock/b200/row_gather.cuh>
 
 namespace gunrock {
 namespace bc {
 namespace detail {
 using b200::counter_t;
 
-constexpr int short_degree = 8;   // below: one thread per row
-constexpr int hub_degree = 4096;  // from here: one CTA per row
 constexpr int buckets_per_level = 9;
-
-__device__ __forceinline__ int degree_bin(long long degree) {
-  return degree < short_degree ? 0 : degree < hub_degree ? 1 : 2;
-}
 
 /// Bucket of vertex v (-1 when unreached), and the edges the two gathers walk for it (in-edges except at the source's
 /// level, out-edges always). `bad` counts depths at or beyond `levels`, which a BFS result never has.
@@ -75,7 +71,7 @@ __device__ __forceinline__ long long bucket_of(std::size_t v, std::size_t n, con
   const long long in_deg = (long long)(in_offsets[v + 1] - in_offsets[v]);
   const long long out_deg = (long long)(out_offsets[v + 1] - out_offsets[v]);
   edges += (unsigned long long)((d > 0 ? in_deg : 0) + out_deg);
-  return (long long)d * buckets_per_level + 3 * degree_bin(in_deg) + degree_bin(out_deg);
+  return (long long)d * buckets_per_level + 3 * b200::degree_bin(in_deg) + b200::degree_bin(out_deg);
 }
 
 /// hist[bucket] += vertices in it (one atomic per distinct bucket per warp); stats[0] += edges both gathers will
@@ -142,37 +138,30 @@ __global__ void __launch_bounds__(256)
   }
 }
 
-/// Up to three runs of the level order walked as one row list: a backward level's rows of one out-degree bin lie in
-/// three buckets, one per in-degree bin; a forward level's rows of one in-degree bin are one run.
-struct runs_t {
-  counter_t begin[3];
-  counter_t size[3];
-  __device__ __forceinline__ counter_t at(counter_t i) const {
-    if (i < size[0]) return begin[0] + i;
-    i -= size[0];
-    if (i < size[1]) return begin[1] + i;
-    return begin[2] + (i - size[1]);
-  }
-};
-
 /// Σ value[x] over the list entries x of [first, end) (stride `step`) with depth[x] == want; depth is read first.
 template <typename vertex_t, typename edge_t>
-__device__ __forceinline__ double sum_level(const vertex_t* __restrict__ indices, edge_t first, edge_t end, edge_t step,
-                                            const vertex_t* __restrict__ depth, vertex_t want,
-                                            const double* __restrict__ value) {
-  double acc = 0;
-  for (edge_t e = first; e < end; e += step) {
-    const vertex_t x = __ldg(indices + e);
-    if (__ldg(depth + x) == want) acc = __dadd_rn(acc, __ldg(value + x));
+struct level_sum_t {
+  const vertex_t* indices;
+  const vertex_t* depth;
+  vertex_t want;
+  const double* value;
+  __device__ __forceinline__ double operator()(edge_t first, edge_t end, edge_t step) const {
+    double acc = 0;
+    for (edge_t e = first; e < end; e += step) {
+      const vertex_t x = __ldg(indices + e);
+      if (__ldg(depth + x) == want) acc = __dadd_rn(acc, __ldg(value + x));
+    }
+    return acc;
   }
-  return acc;
-}
+};
 
 /// Forward finish: σ(v) = the sum over the in-edges from the previous level.
 template <typename vertex_t>
 struct forward_t {
   double* sigma;
+  __device__ __forceinline__ void start() {}
   __device__ __forceinline__ void operator()(vertex_t v, double sum) const { sigma[v] = sum; }
+  __device__ __forceinline__ void flush() {}
 };
 
 /// Backward finish: δ(v) = σ(v) · Σ c(w), c(v) = (1 + δ(v)) / σ(v), acc[v] += δ(v) unless v is the source.
@@ -182,55 +171,15 @@ struct backward_t {
   double* c;
   double* acc;
   vertex_t source;
+  __device__ __forceinline__ void start() {}
   __device__ __forceinline__ void operator()(vertex_t v, double sum) const {
     const double s = sigma[v];
     const double delta = __dmul_rn(s, sum);
     c[v] = __ddiv_rn(__dadd_rn(1.0, delta), s);
     if (v != source) acc[v] = __dadd_rn(acc[v], delta);
   }
+  __device__ __forceinline__ void flush() {}
 };
-
-/// mode 0: one thread per listed row; 1: one warp per row; 2: one CTA (256 threads) per row. Each row v of `rows`
-/// gets finish(v, Σ value[x] over its list entries x with depth[x] == want). The lanes of a warp or CTA stride the list
-/// and their partial sums are reduced in a fixed tree, so every sum's order depends on the row's degree alone.
-template <int mode, typename vertex_t, typename edge_t, typename finish_t>
-__global__ void __launch_bounds__(256)
-    level_gather_kernel(const edge_t* __restrict__ offsets, const vertex_t* __restrict__ indices,
-                        const vertex_t* __restrict__ order, runs_t rows, counter_t n_rows,
-                        const vertex_t* __restrict__ depth, vertex_t want, const double* value, finish_t finish) {
-  if constexpr (mode == 0) {
-    for (counter_t i = counter_t(blockIdx.x) * blockDim.x + threadIdx.x; i < n_rows;
-         i += counter_t(gridDim.x) * blockDim.x) {
-      const vertex_t v = order[rows.at(i)];
-      finish(v, sum_level(indices, offsets[v], offsets[v + 1], edge_t(1), depth, want, value));
-    }
-  } else if constexpr (mode == 1) {
-    const unsigned lane = b200::lane_id();
-    const counter_t warps = (counter_t(gridDim.x) * blockDim.x) >> 5;
-    for (counter_t i = (counter_t(blockIdx.x) * blockDim.x + threadIdx.x) >> 5; i < n_rows; i += warps) {
-      const vertex_t v = order[rows.at(i)];
-      double acc = sum_level(indices, edge_t(offsets[v] + lane), offsets[v + 1], edge_t(32), depth, want, value);
-      acc = b200::warp_sum(acc);
-      if (lane == 0) finish(v, acc);
-    }
-  } else {
-    __shared__ double block_acc[256 / 32];
-    for (counter_t i = blockIdx.x; i < n_rows; i += gridDim.x) {
-      const vertex_t v = order[rows.at(i)];
-      double acc = sum_level(indices, edge_t(offsets[v] + threadIdx.x), offsets[v + 1], edge_t(256), depth, want,
-                             value);
-      acc = b200::warp_sum(acc);
-      if (b200::lane_id() == 0) block_acc[threadIdx.x >> 5] = acc;
-      __syncthreads();
-      if (threadIdx.x == 0) {
-        double total = 0;
-        for (int k = 0; k < 256 / 32; ++k) total = __dadd_rn(total, block_acc[k]);
-        finish(v, total);
-      }
-      __syncthreads();
-    }
-  }
-}
 
 template <typename weight_t>
 __global__ void __launch_bounds__(256)
@@ -240,27 +189,6 @@ __global__ void __launch_bounds__(256)
     out[v] = weight_t(__dmul_rn(scale, acc[v]));
 }
 
-/// The three launches of one gather level, one per degree bin, skipping empty bins.
-template <typename vertex_t, typename edge_t, typename finish_t>
-void gather_level(gcuda::standard_context_t& ctx, const graph::adjacency_t<vertex_t, edge_t, float>& A,
-                  const vertex_t* order, const runs_t (&rows)[3], const vertex_t* depth, vertex_t want,
-                  const double* value, finish_t finish) {
-  auto stream = ctx.stream();
-  for (int mode = 0; mode < 3; ++mode) {
-    const counter_t n_rows = rows[mode].size[0] + rows[mode].size[1] + rows[mode].size[2];
-    if (!n_rows) continue;
-    if (mode == 0)
-      level_gather_kernel<0><<<b200::stream_grid(ctx, n_rows), 256, 0, stream>>>(
-          A.offsets, A.indices, order, rows[mode], n_rows, depth, want, value, finish);
-    else if (mode == 1)
-      level_gather_kernel<1><<<gcuda::persistent_grid(ctx, (n_rows + 7) / 8, 8), 256, 0, stream>>>(
-          A.offsets, A.indices, order, rows[mode], n_rows, depth, want, value, finish);
-    else
-      level_gather_kernel<2><<<gcuda::persistent_grid(ctx, n_rows, 8), 256, 0, stream>>>(
-          A.offsets, A.indices, order, rows[mode], n_rows, depth, want, value, finish);
-    ctx.profiler().launches_total += 1;
-  }
-}
 }  // namespace detail
 
 /**
@@ -277,7 +205,7 @@ float run(graph_t& G, const typename graph_t::vertex_type* sources, std::size_t 
   using vertex_t = typename graph_t::vertex_type;
   using edge_t = typename graph_t::edge_type;
   using detail::counter_t;
-  using detail::runs_t;
+  using runs_t = b200::row_runs_t<vertex_t>;
   constexpr int B = detail::buckets_per_level;
 
   error::throw_if_exception(bc_values == nullptr, "bc::run: bc_values is required");
@@ -347,19 +275,20 @@ float run(graph_t& G, const typename graph_t::vertex_type* sources, std::size_t 
     for (int d = 1; d <= deepest; ++d) {  // rows of one in-degree bin: one run of three buckets
       runs_t rows[3];
       for (int t = 0; t < 3; ++t)
-        rows[t] = runs_t{{bucket(d, 3 * t), 0, 0}, {bucket(d, 3 * t + 3) - bucket(d, 3 * t), 0, 0}};
-      detail::gather_level(*ctx, in_view, order.data(), rows, depth.data(), vertex_t(d - 1), sigma.data(),
-                           detail::forward_t<vertex_t>{sigma.data()});
+        rows[t] = runs_t{{order.data() + bucket(d, 3 * t)}, {bucket(d, 3 * t + 3) - bucket(d, 3 * t)}};
+      const detail::level_sum_t<vertex_t, edge_t> sum{in_view.indices, depth.data(), vertex_t(d - 1), sigma.data()};
+      b200::row_gather(*ctx, in_view.offsets, rows, sum, detail::forward_t<vertex_t>{sigma.data()});
     }
     for (int d = deepest; d >= 0; --d) {  // rows of one out-degree bin: one bucket per in-degree bin
       runs_t rows[3];
       for (int t = 0; t < 3; ++t)
         for (int k = 0; k < 3; ++k) {
-          rows[t].begin[k] = bucket(d, 3 * k + t);
+          rows[t].begin[k] = order.data() + bucket(d, 3 * k + t);
           rows[t].size[k] = bucket(d, 3 * k + t + 1) - bucket(d, 3 * k + t);
         }
-      detail::gather_level(*ctx, out_view, order.data(), rows, depth.data(), vertex_t(d + 1), c.data(),
-                           detail::backward_t<vertex_t>{sigma.data(), c.data(), acc.data(), s});
+      const detail::level_sum_t<vertex_t, edge_t> sum{out_view.indices, depth.data(), vertex_t(d + 1), c.data()};
+      b200::row_gather(*ctx, out_view.offsets, rows, sum,
+                       detail::backward_t<vertex_t>{sigma.data(), c.data(), acc.data(), s});
     }
     error::check_last("bc::run gathers");
   }

@@ -17,6 +17,7 @@
 #pragma once
 
 #include <gunrock/algorithms/algorithms.hxx>
+#include <gunrock/b200/row_gather.cuh>
 
 namespace gunrock {
 namespace pr {
@@ -97,11 +98,8 @@ __global__ void __launch_bounds__(256)
   if (b200::lane_id() == 0 && mine != 0) atomicAdd(dangling, mine);
 }
 
-/// Rows binned once per graph by in-degree: [0, short_degree) one thread each, [short_degree, hub_degree) one
-/// warp each, the rest one CTA each. Lists are ascending (stable) so neighbouring threads touch neighbouring rows.
-constexpr int short_degree = 8;
-constexpr int hub_degree = 4096;
-
+/// Rows binned once per graph by in-degree into the three lists of b200::row_gather (see b200::degree_bin). Lists are
+/// ascending (stable) so neighbouring threads touch neighbouring rows.
 template <typename vertex_t, typename edge_t>
 __global__ void __launch_bounds__(256)
     bin_rows_kernel(const edge_t* __restrict__ offsets, vertex_t n, vertex_t* __restrict__ short_rows,
@@ -109,83 +107,56 @@ __global__ void __launch_bounds__(256)
   for (std::size_t base = std::size_t(blockIdx.x) * blockDim.x; base < std::size_t(n);
        base += std::size_t(gridDim.x) * blockDim.x) {
     const std::size_t v = base + threadIdx.x;
-    long long d = -1;
-    if (v < std::size_t(n)) d = (long long)(offsets[v + 1] - offsets[v]);
-    const bool is_short = d >= 0 && d < short_degree, is_hub = d >= hub_degree, is_warp = d >= short_degree && !is_hub;
-    counter_t at = b200::warp_append_slot(is_short, counts + 0);
-    if (is_short) short_rows[at] = vertex_t(v);
-    at = b200::warp_append_slot(is_warp, counts + 1);
-    if (is_warp) warp_rows[at] = vertex_t(v);
-    at = b200::warp_append_slot(is_hub, counts + 2);
-    if (is_hub) hub_rows[at] = vertex_t(v);
+    const int bin = v < std::size_t(n) ? b200::degree_bin((long long)(offsets[v + 1] - offsets[v])) : -1;
+    counter_t at = b200::warp_append_slot(bin == 0, counts + 0);
+    if (bin == 0) short_rows[at] = vertex_t(v);
+    at = b200::warp_append_slot(bin == 1, counts + 1);
+    if (bin == 1) warp_rows[at] = vertex_t(v);
+    at = b200::warp_append_slot(bin == 2, counts + 2);
+    if (bin == 2) hub_rows[at] = vertex_t(v);
   }
 }
 
-/// Σ over the in-edges [beg, end) strided by `step` starting at `first`, double accumulator.
+/// Σ contrib[u]·w over the in-edges [first, end) of a row, strided by `step`, double accumulator.
 template <typename vertex_t, typename edge_t, typename weight_t>
-__device__ __forceinline__ double gather_edges(const graph::adjacency_t<vertex_t, edge_t, weight_t>& A,
-                                               const weight_t* __restrict__ contrib, edge_t first, edge_t end,
-                                               edge_t step) {
-  double acc = 0;
-  if (A.values) {
-    for (edge_t e = first; e < end; e += step) acc += double(__ldg(contrib + __ldg(A.indices + e)) * __ldg(A.values + e));
-  } else {
-    for (edge_t e = first; e < end; e += step) acc += double(__ldg(contrib + __ldg(A.indices + e)));
+struct in_edge_sum_t {
+  const vertex_t* indices;
+  const weight_t* values;  ///< null: weight 1
+  const weight_t* contrib;
+  __device__ __forceinline__ double operator()(edge_t first, edge_t end, edge_t step) const {
+    double acc = 0;
+    if (values) {
+      for (edge_t e = first; e < end; e += step) acc += double(__ldg(contrib + __ldg(indices + e)) * __ldg(values + e));
+    } else {
+      for (edge_t e = first; e < end; e += step) acc += double(__ldg(contrib + __ldg(indices + e)));
+    }
+    return acc;
   }
-  return acc;
-}
+};
 
-template <typename weight_t>
-__device__ __forceinline__ void finish_row(weight_t* p, const weight_t* plast, std::size_t v, double base, double acc,
-                                           float& err) {
-  const weight_t x = weight_t(base + acc);
-  p[v] = x;
-  err = fmaxf(err, fabsf(float(x) - float(plast[v])));
-}
-
-/// mode 0: one thread per listed row; 1: one warp per row; 2: one CTA per row. p[v] = base + Σ contrib·w (pull
-/// PageRank), and the convergence error max|p - plast| is folded in (no separate pass).
-template <int mode, typename vertex_t, typename edge_t, typename weight_t>
-__global__ void __launch_bounds__(256)
-    gather_rows_kernel(const graph::adjacency_t<vertex_t, edge_t, weight_t> A, const vertex_t* __restrict__ rows,
-                       std::size_t n_rows, const weight_t* __restrict__ contrib, const weight_t* __restrict__ plast,
-                       weight_t* __restrict__ p, weight_t alpha, const double* dangling, unsigned* err_bits) {
-  __shared__ double block_acc[256 / 32];
-  const double base = (1.0 - double(alpha) + *dangling) / double(A.n);
-  const unsigned lane = b200::lane_id();
+/// p[v] = base + Σ with base = (1 - alpha + dangling) / n read once per thread, and the convergence error
+/// max|p - plast| folded in (no separate pass): flush() takes the warp's maximum into *err_bits.
+template <typename vertex_t, typename weight_t>
+struct pull_finish_t {
+  weight_t* p;
+  const weight_t* plast;
+  const double* dangling;
+  weight_t alpha;
+  vertex_t n;
+  unsigned* err_bits;
+  double base;
   float err = 0.f;
-  if constexpr (mode == 0) {
-    for (std::size_t i = std::size_t(blockIdx.x) * blockDim.x + threadIdx.x; i < n_rows;
-         i += std::size_t(gridDim.x) * blockDim.x) {
-      const vertex_t v = rows[i];
-      finish_row(p, plast, std::size_t(v), base, gather_edges(A, contrib, A.offsets[v], A.offsets[v + 1], edge_t(1)), err);
-    }
-  } else if constexpr (mode == 1) {
-    const std::size_t warps = (std::size_t(gridDim.x) * blockDim.x) >> 5;
-    for (std::size_t i = (std::size_t(blockIdx.x) * blockDim.x + threadIdx.x) >> 5; i < n_rows; i += warps) {
-      const vertex_t v = rows[i];
-      double acc = gather_edges(A, contrib, edge_t(A.offsets[v] + lane), A.offsets[v + 1], edge_t(32));
-      acc = b200::warp_sum(acc);
-      if (lane == 0) finish_row(p, plast, std::size_t(v), base, acc, err);
-    }
-  } else {
-    for (std::size_t i = blockIdx.x; i < n_rows; i += gridDim.x) {
-      const vertex_t v = rows[i];
-      double acc = gather_edges(A, contrib, edge_t(A.offsets[v] + threadIdx.x), A.offsets[v + 1], edge_t(256));
-      acc = b200::warp_sum(acc);
-      if (lane == 0) block_acc[threadIdx.x >> 5] = acc;
-      __syncthreads();
-      if (threadIdx.x == 0) {
-        double total = 0;
-        for (int k = 0; k < 256 / 32; ++k) total += block_acc[k];
-        finish_row(p, plast, std::size_t(v), base, total, err);
-      }
-      __syncthreads();
-    }
+  __device__ __forceinline__ void start() { base = (1.0 - double(alpha) + *dangling) / double(n); }
+  __device__ __forceinline__ void operator()(vertex_t v, double sum) {
+    const weight_t x = weight_t(base + sum);
+    p[v] = x;
+    err = fmaxf(err, fabsf(float(x) - float(plast[v])));
   }
-  err = b200::warp_max(err);
-  if (lane == 0 && err > 0.f) atomicMax(err_bits, __float_as_uint(err));
-}
+  __device__ __forceinline__ void flush() {
+    err = b200::warp_max(err);
+    if (b200::lane_id() == 0 && err > 0.f) atomicMax(err_bits, __float_as_uint(err));
+  }
+};
 }  // namespace kernels
 
 template <typename graph_t, typename param_type, typename result_type>
@@ -203,7 +174,7 @@ struct problem_t : gunrock::problem_t<graph_t> {
   bool pull = false;
   memory::device_array_t<weight_t> contrib;
   memory::device_array_t<vertex_t> short_rows, warp_rows, hub_rows;
-  std::size_t n_short = 0, n_warp = 0, n_hub = 0;
+  b200::row_runs_t<vertex_t> rows[3] = {};  ///< the three lists as b200::row_gather walks them
 
   problem_t(graph_t& G, param_type& _param, result_type& _result, std::shared_ptr<gcuda::multi_context_t> _context)
       : gunrock::problem_t<graph_t>(G, _context), param(_param), result(_result) {}
@@ -237,7 +208,9 @@ struct problem_t : gunrock::problem_t<graph_t> {
     b200::counter_t h[3] = {0, 0, 0};
     cudaMemcpyAsync(h, counts.data(), sizeof(h), cudaMemcpyDeviceToHost, ctx->stream());
     ctx->synchronize();
-    n_short = std::size_t(h[0]), n_warp = std::size_t(h[1]), n_hub = std::size_t(h[2]);
+    rows[0] = {{short_rows.data()}, {h[0]}};
+    rows[1] = {{warp_rows.data()}, {h[1]}};
+    rows[2] = {{hub_rows.data()}, {h[2]}};
   }
   void reset() override {
     auto* ctx = this->get_single_context();
@@ -285,15 +258,9 @@ struct enactor_t : gunrock::enactor_t<problem_t> {
       unsigned* err_bits = reinterpret_cast<unsigned*>(P->scalars.data() + 1);
       kernels::snapshot_contrib_kernel<<<b200::stream_grid(*ctx, n), 256, 0, ctx->stream()>>>(p, plast, iweights, contrib,
                                                                                               n, alpha, dangling);
-      if (P->n_short)
-        kernels::gather_rows_kernel<0><<<b200::stream_grid(*ctx, P->n_short), 256, 0, ctx->stream()>>>(
-            A, P->short_rows.data(), P->n_short, contrib, plast, p, alpha, dangling, err_bits);
-      if (P->n_warp)
-        kernels::gather_rows_kernel<1><<<gcuda::persistent_grid(*ctx, (P->n_warp + 7) / 8, 8), 256, 0, ctx->stream()>>>(
-            A, P->warp_rows.data(), P->n_warp, contrib, plast, p, alpha, dangling, err_bits);
-      if (P->n_hub)
-        kernels::gather_rows_kernel<2><<<gcuda::persistent_grid(*ctx, P->n_hub, 8), 256, 0, ctx->stream()>>>(
-            A, P->hub_rows.data(), P->n_hub, contrib, plast, p, alpha, dangling, err_bits);
+      b200::row_gather(*ctx, A.offsets, P->rows,
+                       kernels::in_edge_sum_t<vertex_t, edge_t, weight_t>{A.indices, A.values, contrib},
+                       kernels::pull_finish_t<vertex_t, weight_t>{p, plast, dangling, alpha, A.n, err_bits});
       error::check_last("pr gather");
       (void)spread;
       (void)E;

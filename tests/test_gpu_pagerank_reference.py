@@ -19,7 +19,7 @@ pytestmark = pytest.mark.gpu
 LBS = list(ess.IMPLEMENTED_LOAD_BALANCERS)
 ALPHA = float(np.float32(0.85))  # the kernels compute with the float alpha
 KNOB_DEFAULTS = {"advance_engine": 1}
-HUB_DEGREE = 4096  # pr::kernels::hub_degree (one CTA per row) and advance kernels::big_degree (grid-wide)
+HUB_DEGREE = 4096  # b200::hub_degree (one CTA per row) and advance kernels::big_degree (grid-wide)
 IN_HUB_DEGREES = (7, 8, 4095, 4096, 4097, 9001)
 OUT_HUB_DEGREES = (4096, 6007)
 
